@@ -5,7 +5,7 @@ Metric (BASELINE.json): QPS at recall@10 >= 0.95 on 1M x 768 fp32 cosine (config
 HNSW build vectors/s and, at every N, the hash-partitioned search (configs[2]) and build (configs[3]).
 One "step" = one pass of the batched scan (hnswgettuple for nq queries) over one batch of synthetic queries.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   torchrun ... bench.py --gpus N ...        (one rank per GPU)
 
 The one JSON line:
@@ -20,6 +20,12 @@ The one JSON line:
                            in a CHILD PROCESS that maps neither CUDA nor the product library, on the graph the GPU
                            built; its ids for the same queries are compared with the GPU's.
 `--workload partitioned|build` print a line for those shapes alone.
+
+`--dump-outputs DIR` (configs[1]): after the timed steps, rank 0 writes what the last timed step's scan returned
+as DIR/elements.npy (element ids, -1 past the count), DIR/distances.npy (+inf past the count) and DIR/counts.npy,
+one row per query, plus DIR/rows.npy (the query rows written).  Ids and counts are stored as float64, which holds
+them exactly; distances as float32.  Above 64 MB in all, a fixed seeded sample of the queries is written.  Inputs
+depend on the arguments only, so two builds of the project can be compared output for output.
 
 `--impl reference`: the reference's CPU path.  The mount has no source and there is no PostgreSQL
 (/root/reference/README.md:1), so what is timed is the C oracle (oracle/, "CPU restatement of pgvector HNSW
@@ -136,6 +142,27 @@ def exact_topk_metric(x_dev, q_dev, k, metric):
 
 def recall_at(ids, gt):
     return float(np.mean([len(set(ids[i]) & set(gt[i])) / gt.shape[1] for i in range(gt.shape[0])]))
+
+
+DUMP_LIMIT = 64 * 10 ** 6
+
+
+def dump_outputs(d, arrays, limit=DUMP_LIMIT):
+    """Writes arrays that share a first axis (one row per query) as d/<name>.npy: integers as float64 (exact up to
+    2**53), floats as float32.  When the files would exceed `limit` bytes, the same fixed seeded sample of rows is
+    written from every array.  d/rows.npy lists the rows written."""
+    arrays = {k: np.asarray(a, np.float64 if np.issubdtype(np.asarray(a).dtype, np.integer) else np.float32)
+              for k, a in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    per_row = 8 + sum(a[:1].nbytes for a in arrays.values())
+    budget = limit - 1024 * (len(arrays) + 1)          # .npy headers
+    rows = np.arange(n)
+    if n * per_row > budget:
+        rows = np.sort(np.random.default_rng(0).choice(n, budget // per_row, replace=False))
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "rows.npy"), rows.astype(np.float64))
+    for k, a in arrays.items():
+        np.save(os.path.join(d, k + ".npy"), a[rows])
 
 
 class ClockSampler:
@@ -316,7 +343,13 @@ def main():
     ap.add_argument("--cpu-budget", type=float, default=20.0, help="seconds of CPU work for the search baseline")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sub", action="store_true", help="skip the partitioned / build_partitioned sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's scan outputs as DIR/<name>.npy (configs[1], --impl ours)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c2"):
+        ap.error("--dump-outputs writes the configs[1] scan of --impl ours")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -445,6 +478,10 @@ def main():
     total_ms = ev0.elapsed_time(ev1)
     ctr = ix.counters(reset=True)
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        # before the single launch below, which writes slot 0 again
+        dump_outputs(args.dump_outputs, dict(zip(("elements", "distances", "counts"),
+                                                 (t.cpu().numpy() for t in outs[(args.steps - 1) % NSLOT]))))
     if world > 1:
         t = torch.tensor([total_ms], device=dev)
         torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)

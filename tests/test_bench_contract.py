@@ -92,3 +92,39 @@ def test_cpu_arm_child_process(tmp_path):
     bd[0, 0] = od[0, 20]
     rec2 = bench.parity_record(par, bad, bd)
     assert rec2["canonical_order"]["ids_identical"] == 99 and rec2["natural_order_top10"]["unexplained"] == 1
+
+
+def test_dump_outputs_writes_float_arrays_and_samples_above_the_limit(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    elem = np.arange(60, dtype=np.int32).reshape(20, 3)
+    elem[4, 2] = -1
+    dist = (elem / 7).astype(np.float32)
+    dist[4, 2] = np.inf
+    arrays = {"elements": elem, "distances": dist, "counts": np.full(20, 3, np.int32)}
+    d = str(tmp_path / "all")
+    bench.dump_outputs(d, arrays)
+    got = {k: np.load(os.path.join(d, k + ".npy")) for k in ("elements", "distances", "counts", "rows")}
+    assert got["elements"].dtype == np.float64 and got["counts"].dtype == np.float64 and got["distances"].dtype == np.float32
+    assert (got["rows"] == np.arange(20)).all() and (got["elements"] == elem).all() and (got["counts"] == 3).all()
+    assert (got["distances"].view(np.uint32) == dist.view(np.uint32)).all()
+    # 52 bytes a row (rows + 3 ids + 3 distances + count) and 1 kB per header: room for 10 of the 20 rows
+    limit = 4 * 1024 + 52 * 10
+    picks = []
+    for tag in ("a", "b"):
+        d = str(tmp_path / tag)
+        bench.dump_outputs(d, arrays, limit=limit)
+        rows = np.load(os.path.join(d, "rows.npy")).astype(np.int64)
+        assert len(rows) == 10 and (np.diff(rows) > 0).all()
+        assert (np.load(os.path.join(d, "elements.npy")) == elem[rows]).all()
+        assert (np.load(os.path.join(d, "distances.npy")).view(np.uint32) == dist[rows].view(np.uint32)).all()
+        assert sum(os.path.getsize(os.path.join(d, f)) for f in os.listdir(d)) <= limit
+        picks.append(rows)
+    assert (picks[0] == picks[1]).all()
+
+
+def test_dump_outputs_is_refused_outside_the_headline_scan(tmp_path):
+    for extra in (["--impl", "reference"], ["--workload", "build"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--dump-outputs", str(tmp_path)] + extra,
+                             capture_output=True, text=True, timeout=300)
+        assert out.returncode == 2 and "--dump-outputs" in out.stderr and out.stdout == ""
