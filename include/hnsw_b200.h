@@ -123,7 +123,9 @@ int hb_set_option(hb_index *ix, const char *name, int value);
 /* ---- flat graph image (the layout in HBM; DESIGN.md "Data layout") ------------------------- */
 /* Load a graph built elsewhere (e.g. by the CPU oracle, or converted from pgvector index pages).
  * vecs n x dim (normalised already when cosine); level n; nbr0 n x 2m (-1 pad); uoff n (row into
- * nbru or -1); nbru upper_rows x m; ntids n (NULL = all 1); tids n x HB_HEAPTIDS (NULL = id). */
+ * nbru or -1); nbru upper_rows x m; ntids n (NULL = all 1); tids n x HB_HEAPTIDS (NULL = id).
+ * entry -1 with n > 0 (no entry point) is accepted only when no element holds a heap TID: the state vacuum
+ * leaves after removing every element; the next insert becomes the entry point. */
 int hb_index_load(hb_index *ix, int64_t n, int64_t upper_rows, int32_t entry, const void *vecs,
                   const uint8_t *level, const int32_t *nbr0, const int32_t *uoff,
                   const int32_t *nbru, const uint8_t *ntids, const int64_t *tids);
@@ -131,7 +133,7 @@ int hb_index_load(hb_index *ix, int64_t n, int64_t upper_rows, int32_t entry, co
  * x 8192 bytes: block 0 = metapage, then element / neighbour tuples; pgvector 0.7-0.8 layout AS
  * RECALLED -- see csrc/pgpages.cu).  The handle's dim, m and dtype must match the index; vectors of
  * a cosine index are stored normalised already.  Deleted elements keep their place in the graph
- * and return no tuples. */
+ * and return no tuples; a metapage without an entry point loads as hb_index_load's entry -1. */
 int hb_index_load_pgvector_pages(hb_index *ix, const void *pages, int64_t n_pages);
 /* what the pages hold (metapage fields, element and upper-layer row counts) -- to size hb_index_create;
  * host only, needs no device; any out pointer may be NULL */

@@ -56,6 +56,7 @@ struct OrcIndex {
     uint8_t *ntids; int64_t *tids;                      /* n x ORC_HEAPTIDS */
     uint8_t *deleted;                                   /* HnswElementTupleData.deleted (set by vacuum's MarkDeleted) */
     int32_t entry; int entry_level;
+    int stale_d;               /* cached distances unknown (imported graph): recomputed before the next insert */
     OrcCounters ctr;
 };
 
@@ -580,9 +581,25 @@ static void grow_upper(OrcIndex *ix, int64_t need)
 
 /* ------------------------------------------------------------------ insert (in-memory build) */
 
+/* an imported graph carries no owner->neighbour distances: compute them as the first insert needs them (the GPU
+ * library does the same for a loaded graph) */
+static void refresh_cached_distances(OrcIndex *ix)
+{
+    int m2 = 2 * ix->m, m = ix->m;
+    for (int64_t e = 0; e < ix->n; e++) {
+        for (int i = 0; i < ix->cnt0[e]; i++) ix->nbr0d[e * m2 + i] = dist_elems(ix, e, ix->nbr0[e * m2 + i], NULL);
+        for (int l = 1; l <= ix->level[e]; l++) {
+            int64_t r = (int64_t) ix->uoff[e] + l - 1;
+            for (int i = 0; i < ix->cntu[r]; i++) ix->nbrud[r * m + i] = dist_elems(ix, e, ix->nbru[r * m + i], NULL);
+        }
+    }
+    ix->stale_d = 0;
+}
+
 int64_t orc_insert(OrcIndex *ix, const void *vec, int64_t heap_tid)
 {
     int dim = ix->dim;
+    if (ix->stale_d) refresh_cached_distances(ix);
     size_t rowb = (size_t) dim * ix->esize;
     grow_elems(ix, ix->n + 1);
     int64_t e = ix->n;
@@ -1180,5 +1197,6 @@ OrcIndex *orc_import(int dim, int m, int efc, int metric, int dtype, int dist_mo
     }
     ix->n = n; ix->urows = upper_rows; ix->seq = n;
     ix->entry = entry; ix->entry_level = entry >= 0 ? level[entry] : -1;
+    ix->stale_d = 1;
     return ix;
 }

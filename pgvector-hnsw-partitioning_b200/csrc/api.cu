@@ -500,7 +500,15 @@ int hb_index_load(hb_index *ix, int64_t n, int64_t upper_rows, int32_t entry, co
         set_error("hb_index_load: graph (%lld elements, %lld upper rows) exceeds capacity", (long long) n, (long long) upper_rows);
         return HB_ENOMEM;
     }
-    if (n > 0 && (entry < 0 || entry >= n)) { set_error("hb_index_load: entry point %d is not an element (n = %lld)", entry, (long long) n); return HB_EINVAL; }
+    if (n > 0 && (entry < -1 || entry >= n)) { set_error("hb_index_load: entry point %d is not an element (n = %lld)", entry, (long long) n); return HB_EINVAL; }
+    // no entry point with elements present: what vacuum leaves when it removed every element; only then
+    if (n > 0 && entry < 0) {
+        for (int64_t e = 0; e < n; e++)
+            if (!ntids || ntids[e] > 0) {
+                set_error("hb_index_load: no entry point, but element %lld holds heap TIDs", (long long) e);
+                return HB_EINVAL;
+            }
+    }
     for (int64_t i = 0; i < n * 2 * ix->m; i++)
         if (nbr0[i] < -1 || nbr0[i] >= n) { set_error("hb_index_load: layer-0 neighbour id %d out of range", nbr0[i]); return HB_EINVAL; }
     for (int64_t i = 0; i < upper_rows * ix->m; i++)

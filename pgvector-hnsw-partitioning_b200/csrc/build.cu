@@ -460,8 +460,9 @@ int64_t build_insert(hb_index *ix, const void *host_vecs, int64_t n_in, const in
         b = std::min<int64_t>(b, (int64_t) todo.size() - pos);
         levels.resize(b);
         for (int64_t i = 0; i < b; i++) levels[i] = (uint8_t) level_for(ix->seed, ix->seq + i, m);
-        // an element above the current entry level becomes the entry point: insert it alone
-        if (cur > 0) {
+        // an element above the current entry level becomes the entry point: insert it alone; so does the first element
+        // of a graph without an entry point (empty, or every element vacuumed away)
+        if (ix->entry >= 0) {
             if (levels[0] > ix->entry_level) b = 1;
             else for (int64_t i = 1; i < b; i++) if (levels[i] > ix->entry_level) { b = i; break; }
         } else b = 1;
@@ -475,33 +476,52 @@ int64_t build_insert(hb_index *ix, const void *host_vecs, int64_t n_in, const in
 
         auto tid_of = [&](int64_t i) { return heap_tids ? heap_tids[todo[pos + i]] : todo[pos + i]; };
 
-        if (cur == 0) {
-            // first element: becomes the entry point, no neighbours
+        if (ix->entry < 0) {
+            // first element of a graph without an entry point: slot cur (elements vacuumed away keep theirs), no
+            // neighbours; it becomes the entry point
             const int lv = levels[0];
-            if (lv > ix->upper_cap) { set_error("upper layer table full"); return HB_ENOMEM; }   // cannot happen: upper_cap >= 1024
-            int32_t uo = lv > 0 ? 0 : -1;
-            HB_CK(cudaMemcpyAsync(ix->d_uoff, &uo, sizeof uo, cudaMemcpyHostToDevice, s));
+            const int64_t ur = ix->upper_rows;
+            if (ur + lv > ix->upper_cap) {
+                if (!ix->opt_auto_grow) { set_error("upper layer table full (%lld rows)", (long long) (ur + lv)); return HB_ENOMEM; }
+                HB_CK(cudaStreamSynchronize(s));
+                HB_CK(cudaStreamSynchronize(up));
+                const int grc = hb_index_reserve(ix, ix->cap + ix->cap / 2 + 1024);
+                if (grc) return grc;
+                uploaded = (int64_t) pos;      // rows uploaded ahead lived in the old array: upload them again
+                slot_base = ix->n - uploaded;
+                continue;
+            }
+            const int64_t t0 = tid_of(0);
+            const int32_t uo = lv > 0 ? (int32_t) ur : -1;
+            const uint8_t one = 1;
+            HB_CK(cudaMemcpyAsync(ix->d_uoff + cur, &uo, sizeof uo, cudaMemcpyHostToDevice, s));
+            HB_CK(cudaMemcpyAsync(ix->d_tid0 + cur, &t0, sizeof t0, cudaMemcpyHostToDevice, s));
+            HB_CK(cudaMemcpyAsync(ix->d_ntids + cur, &one, 1, cudaMemcpyHostToDevice, s));
+            // stale lists and cached distances from a previous life of these rows
+            HB_CK(cudaMemsetAsync(ix->d_nbr0 + (size_t) cur * m2, 0xff, sizeof(int32_t) * m2, s));
+            HB_CK(cudaMemsetAsync(ix->d_nbr0d + (size_t) cur * m2, 0, sizeof(float) * m2, s));
+            if (lv > 0) {
+                HB_CK(cudaMemsetAsync(ix->d_nbru + (size_t) ur * m, 0xff, sizeof(int32_t) * (size_t) lv * m, s));
+                HB_CK(cudaMemsetAsync(ix->d_nbrud + (size_t) ur * m, 0, sizeof(float) * (size_t) lv * m, s));
+            }
+            if (ix->d_pv0) HB_CK(cudaMemsetAsync(ix->d_pv0 + cur, 0, 1, s));
+            if (ix->d_pvu && lv > 0) HB_CK(cudaMemsetAsync(ix->d_pvu + ur, 0, lv, s));
             HB_CK(cudaStreamSynchronize(s));
             ix->h_level.push_back((uint8_t) lv);
             ix->h_ntids.push_back(1);
-            ix->h_tids.resize(HB_HEAPTIDS, 0);
-            ix->h_tids[0] = tid_of(0);
-            ix->upper_rows = lv; ix->n = 1; ix->entry = 0; ix->entry_level = lv; ix->seq += 1;
+            ix->h_tids.resize((size_t) (cur + 1) * HB_HEAPTIDS, 0);
+            ix->h_tids[(size_t) cur * HB_HEAPTIDS] = t0;
+            ix->n = cur + 1; ix->upper_rows = ur + lv;
+            ix->entry = (int32_t) cur; ix->entry_level = lv; ix->seq += 1;
             ix->generation++;
-            // stale lists from a previous life of this slot
-            HB_CK(cudaMemset(ix->d_nbr0, 0xff, sizeof(int32_t) * m2));
-            if (lv > 0) HB_CK(cudaMemset(ix->d_nbru, 0xff, sizeof(int32_t) * (size_t) lv * m));
-            if (ix->d_pv0) HB_CK(cudaMemset(ix->d_pv0, 0, 1));
-            if (ix->d_pvu && lv > 0) HB_CK(cudaMemset(ix->d_pvu, 0, lv));
-            // heap TIDs of the first element
-            {
-                int64_t t0 = ix->h_tids[0];
-                uint8_t one = 1;
-                HB_CK(cudaMemcpy(ix->d_tid0, &t0, sizeof t0, cudaMemcpyHostToDevice));
-                HB_CK(cudaMemcpy(ix->d_ntids, &one, 1, cudaMemcpyHostToDevice));
-            }
             pos += 1; indexed += 1;
             continue;
+        }
+        // the candidate search starts at the entry point: it must be an element (a bad one would be read out of bounds)
+        if (ix->entry >= cur || ix->entry_level < 0) {
+            set_error("insert: entry point %d (level %d) is not an element of the %lld in the graph", ix->entry, ix->entry_level,
+                      (long long) cur);
+            return HB_EINVAL;
         }
 
         // ---- the batch's bookkeeping integers, assuming no tuple folds into a duplicate

@@ -39,14 +39,13 @@ struct RepairParams {
     const uint8_t *ntids;        // per element: 0 = being deleted
     int efc1;                    // ef_construction + 1
     int LS;                      // layer stride of the staging arrays (max level in the batch + 1)
-    int32_t *need;               // B: 1 = new lists staged, 0 = left alone
+    int32_t *need;               // B: 1 = new lists staged, 0 = left alone, -1 = W outgrew gcap (searched again with a larger one)
     int32_t *sel_id; float *sel_d; int32_t *sel_cnt;   // B x LS x lm0, B x LS
     // per-warp scratch in HBM
     uint32_t *gbits; int gwords;
     float *gwd; uint32_t *gwi; int gcap;
     int32_t *c_id; float *c_d; int32_t *wd_id; float *wd_d;   // gcap each per warp
     unsigned int *work;
-    int32_t *err;
     unsigned long long *totals;
     int32_t *nbr0; int32_t *nbru;   // writable views (phase 2)
     int32_t *locks;                  // per element
@@ -220,8 +219,7 @@ __global__ void __launch_bounds__(VAC_WARPS * 32) repair_search_kernel(const Rep
             }
         }
         if (lane == 0) {
-            if (st != ST_OK) atomicExch(p.err, 1);
-            else p.need[i] = 1;
+            p.need[i] = st == ST_OK ? 1 : -1;
             atomicAdd(p.totals + 0, (unsigned long long) ctr.n_dist);
             atomicAdd(p.totals + 1, (unsigned long long) ctr.n_hop0);
             atomicAdd(p.totals + 2, (unsigned long long) ctr.n_hopu);
@@ -252,7 +250,7 @@ __global__ void __launch_bounds__(VAC_WARPS * 32) repair_apply_kernel(const Repa
     unsigned long long npair = 0;
 
     for (int i = blockIdx.x * VAC_WARPS + warp; i < p.B; i += gridDim.x * VAC_WARPS) {
-        if (!p.need[i]) continue;
+        if (p.need[i] != 1) continue;
         const int32_t e = p.elems[i];
         const int level = p.lev[i];
         // the element's own neighbour tuple
@@ -406,10 +404,12 @@ extern "C" int64_t hb_vacuum_repair(hb_index *ix, int64_t *repaired)
     for (int64_t e = 0; e < n; e++) max_level = std::max<int>(max_level, ix->h_level[e]);
     const int LS = max_level + 1;
     const int64_t warps = (int64_t) VAC_GRID * VAC_WARPS;
+    // per-warp W list: ef_construction + 1 + the tie allowance.  Emptied elements stay in W without counting towards
+    // ef, so after heavy deletes a search can outgrow it; such an element is searched again alone with a larger list
     const int gcap = ix->efc + 1 + HB_TIE_LIMIT;
     const int gwords = (int) ((n + 31) / 32 + 1);
-    DevBuf b_elems, b_lev, b_need, b_sel, b_scr, b_misc, b_locks;
-    struct Release { DevBuf *b[7]; ~Release() { for (auto x : b) x->release(); } } rel{ { &b_elems, &b_lev, &b_need, &b_sel, &b_scr, &b_misc, &b_locks } };
+    DevBuf b_elems, b_lev, b_need, b_sel, b_scr, b_misc, b_locks, b_big;
+    struct Release { DevBuf *b[8]; ~Release() { for (auto x : b) x->release(); } } rel{ { &b_elems, &b_lev, &b_need, &b_sel, &b_scr, &b_misc, &b_locks, &b_big } };
     HB_CK(b_elems.ensure(sizeof(int32_t) * (size_t) std::max<int64_t>(bmax, 1)));
     HB_CK(b_lev.ensure((size_t) bmax));
     HB_CK(b_need.ensure(sizeof(int32_t) * (size_t) bmax));
@@ -431,48 +431,72 @@ extern "C" int64_t hb_vacuum_repair(hb_index *ix, int64_t *repaired)
     p.sel_id = b_sel.as<int32_t>();
     p.sel_d = reinterpret_cast<float *>(p.sel_id + (size_t) bmax * LS * lm0);
     p.sel_cnt = reinterpret_cast<int32_t *>(p.sel_d + (size_t) bmax * LS * lm0);
-    {
-        char *c = b_scr.as<char>();
-        p.gbits = reinterpret_cast<uint32_t *>(c); c += (size_t) warps * gwords * 4;
-        p.gwd = reinterpret_cast<float *>(c); c += (size_t) warps * gcap * 4;
-        p.gwi = reinterpret_cast<uint32_t *>(c); c += (size_t) warps * gcap * 4;
-        p.c_id = reinterpret_cast<int32_t *>(c); c += (size_t) warps * gcap * 4;
-        p.c_d = reinterpret_cast<float *>(c); c += (size_t) warps * gcap * 4;
-        p.wd_id = reinterpret_cast<int32_t *>(c); c += (size_t) warps * gcap * 4;
-        p.wd_d = reinterpret_cast<float *>(c);
-    }
-    p.gwords = gwords; p.gcap = gcap;
+    // per-warp scratch of `nw` warps with W lists of `cap` entries
+    auto carve_scratch = [&](RepairParams &q, char *c, int64_t nw, int cap) {
+        q.gbits = reinterpret_cast<uint32_t *>(c); c += (size_t) nw * gwords * 4;
+        q.gwd = reinterpret_cast<float *>(c); c += (size_t) nw * cap * 4;
+        q.gwi = reinterpret_cast<uint32_t *>(c); c += (size_t) nw * cap * 4;
+        q.c_id = reinterpret_cast<int32_t *>(c); c += (size_t) nw * cap * 4;
+        q.c_d = reinterpret_cast<float *>(c); c += (size_t) nw * cap * 4;
+        q.wd_id = reinterpret_cast<int32_t *>(c); c += (size_t) nw * cap * 4;
+        q.wd_d = reinterpret_cast<float *>(c);
+        q.gwords = gwords; q.gcap = cap;
+    };
+    carve_scratch(p, b_scr.as<char>(), warps, gcap);
     unsigned int *misc = b_misc.as<unsigned int>();
     p.work = misc;
-    p.err = reinterpret_cast<int32_t *>(misc + 1);
     p.totals = ix->d_totals;
     p.nbr0 = ix->d_nbr0; p.nbru = ix->d_nbru;
     p.locks = b_locks.as<int32_t>();
 
     std::vector<int32_t> h_need;
     int64_t n_repaired = 0;
-    // one batch: elems through both phases with the given entry point; returns through n_repaired
+    // both phases for elems[0 .. B) with the given entry point and scratch; h_need receives the phase-1 outcome
+    auto launch = [&](RepairParams &q, const int32_t *elems, int B, int32_t entry, int entry_level) -> int {
+        if (entry < -1 || entry >= n) { set_error("hb_vacuum_repair: entry point %d is not an element (n = %lld)", entry, (long long) n); return HB_EINVAL; }
+        std::vector<uint8_t> lev(B);
+        for (int i = 0; i < B; i++) lev[i] = ix->h_level[elems[i]];
+        q.g = ix->view();
+        q.g.entry = entry;
+        q.g.entry_level = entry_level;
+        q.B = B;
+        HB_CK(cudaMemcpyAsync(b_elems.p, elems, sizeof(int32_t) * B, cudaMemcpyHostToDevice, s));
+        HB_CK(cudaMemcpyAsync(b_lev.p, lev.data(), B, cudaMemcpyHostToDevice, s));
+        HB_CK(cudaMemsetAsync(misc, 0, 4, s));
+        const int rc = run_repair(ix, q, s);
+        if (rc) return rc;
+        h_need.resize(B);
+        HB_CK(cudaMemcpyAsync(h_need.data(), b_need.p, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, s));
+        HB_CK(cudaStreamSynchronize(s));
+        return HB_OK;
+    };
+    // one batch through both phases; elements whose W outgrew gcap were left alone by phase 2 and are searched again,
+    // one at a time in element order, on one CTA with W doubled until it fits (W holds distinct elements: n + 1 always does)
     auto run_batch = [&](const std::vector<int32_t> &elems, int32_t entry, int entry_level) -> int {
         const int B = (int) elems.size();
         if (B == 0) return HB_OK;
-        std::vector<uint8_t> lev(B);
-        for (int i = 0; i < B; i++) lev[i] = ix->h_level[elems[i]];
-        p.g = ix->view();
-        p.g.entry = entry;
-        p.g.entry_level = entry_level;
-        p.B = B;
-        HB_CK(cudaMemcpyAsync(b_elems.p, elems.data(), sizeof(int32_t) * B, cudaMemcpyHostToDevice, s));
-        HB_CK(cudaMemcpyAsync(b_lev.p, lev.data(), B, cudaMemcpyHostToDevice, s));
-        HB_CK(cudaMemsetAsync(misc, 0, 4, s));
-        const int rc = run_repair(ix, p, s);
+        int rc = launch(p, elems.data(), B, entry, entry_level);
         if (rc) return rc;
-        h_need.resize(B);
-        int32_t err = 0;
-        HB_CK(cudaMemcpyAsync(h_need.data(), b_need.p, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, s));
-        HB_CK(cudaMemcpyAsync(&err, p.err, sizeof err, cudaMemcpyDeviceToHost, s));
-        HB_CK(cudaStreamSynchronize(s));
-        if (err) { set_error("hb_vacuum_repair: more than %d candidates tie exactly at the ef_construction boundary", HB_TIE_LIMIT); return HB_ELIMIT; }
-        for (int i = 0; i < B; i++) n_repaired += h_need[i];
+        std::vector<int32_t> again;
+        for (int i = 0; i < B; i++) {
+            if (h_need[i] > 0) n_repaired++;
+            else if (h_need[i] < 0) again.push_back(elems[i]);
+        }
+        for (const int32_t e : again) {
+            int cap = gcap;
+            for (;;) {
+                if (cap >= n + 1) {
+                    set_error("hb_vacuum_repair: the repair search of element %d holds more than %d candidates", e, cap);
+                    return HB_ELIMIT;
+                }
+                cap = (int) std::min<int64_t>(2 * (int64_t) cap, n + 1);
+                HB_CK(b_big.ensure((size_t) VAC_WARPS * ((size_t) gwords * 4 + (size_t) cap * 24)));
+                RepairParams q = p;
+                carve_scratch(q, b_big.as<char>(), VAC_WARPS, cap);
+                if ((rc = launch(q, &e, 1, entry, entry_level)) != 0) return rc;
+                if (h_need[0] >= 0) { n_repaired += h_need[0]; break; }
+            }
+        }
         return HB_OK;
     };
 

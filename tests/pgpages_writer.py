@@ -128,9 +128,11 @@ def write_pages(g, m, efc, dim, half=False, scatter=False, deleted=()):
             got = pg.add(bytes(t))
             assert got == off, (got, off)
     meta = bytearray(BLCKSZ)
-    eb, eo = where[int(g.entry)] if n else (INVALID_BLK, 0)
+    # no entry point (an empty index, or one whose every element was vacuumed away): InvalidBlockNumber, offset 0
+    has_entry = n > 0 and int(g.entry) >= 0
+    eb, eo = where[int(g.entry)] if has_entry else (INVALID_BLK, 0)
     struct.pack_into("<QHHHHHHI", meta, 0, 0, 0, 0, 24 + 28, BLCKSZ - 8, BLCKSZ - 8, BLCKSZ | 4, 0)
-    struct.pack_into("<IIIHHIHhI", meta, 24, 0xA953A953, 1, dim, m, efc, eb, eo, int(g.level[int(g.entry)]) if n else -1, len(pages))
+    struct.pack_into("<IIIHHIHhI", meta, 24, 0xA953A953, 1, dim, m, efc, eb, eo, int(g.level[int(g.entry)]) if has_entry else -1, len(pages))
     struct.pack_into("<IHH", meta, BLCKSZ - 8, INVALID_BLK, 0, 0xFF90)
     out = bytes(meta)
     for i, p in enumerate(pages):
