@@ -109,14 +109,14 @@ int hb_set_build_batch(hb_index *ix, int max_batch);
 /* HnswInitElement's level draw for the seq-th initialised element: (int)(-ln(U) / ln(m)), capped */
 int hb_level_for(uint64_t seed, int64_t seq, int m);
 /* tuning knobs: "slots" (visited-table size), "grid" (CTA cap), "build_batch",
- * "per_query_counters" (0/1), "variant" (scan kernel choice, experiments and tests: 0 automatic; 6 never
- * the four-warps-per-query kernels of small batches; 7 / 17 / 27 those kernels for every row length: default form /
- * list in shared memory / no row staging; 10 / 20 the same sub-forms where they are selected anyway; 9 the
- * shared-memory-list warp kernel instead of the register-list one; all give identical results), "link_kernel" (reverse-link
+ * "per_query_counters" (0/1), "variant" (scan kernel forced for tests: 0 automatic; 6 never the
+ * four-warps-per-query kernels of small batches; 7 / 17 / 27 those kernels for every row length: default form /
+ * list in shared memory / no row staging; 9 the shared-memory-list warp kernel instead of the register-list one;
+ * all give identical results; any other value is refused with HB_EINVAL), "link_kernel" (reverse-link
  * kernel: 0 automatic, 1 warp per list, 2 pipelined TMA-staged, 3 memoised pair distances; all give
  * the same graph), "pair_cache" (0 = do not allocate the pair-distance cache), "pair_fill" (0 = fill
- * the cache in place instead of with the pre-pass), "fused_select", "eval_table" (0 = the unfused /
- * recomputing forms of the build kernels), "build_fraction" (a batch is at most 1/value of the graph,
+ * the cache in place instead of with the pre-pass), "eval_table" (0 = the recomputing form of the
+ * reverse-link kernels), "build_fraction" (a batch is at most 1/value of the graph,
  * default 16).  0 restores the automatic choice. */
 int hb_set_option(hb_index *ix, const char *name, int value);
 

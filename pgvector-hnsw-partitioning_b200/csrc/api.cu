@@ -334,11 +334,13 @@ int hb_set_option(hb_index *ix, const char *name, int value)
     else if (!strcmp(name, "grid")) ix->opt_grid = value;
     else if (!strcmp(name, "build_batch")) ix->opt_build_batch = value;
     else if (!strcmp(name, "per_query_counters")) ix->opt_per_query = value;
-    else if (!strcmp(name, "variant")) ix->opt_variant = value;
+    else if (!strcmp(name, "variant")) {
+        if (!is_scan_variant(value)) { set_error("hb_set_option: variant %d is not one of 0, 6, 7, 9, 17, 27", value); return HB_EINVAL; }
+        ix->opt_variant = value;
+    }
     else if (!strcmp(name, "link_kernel")) ix->opt_link_kernel = value;
     else if (!strcmp(name, "pair_cache")) ix->opt_pair_cache = value;
     else if (!strcmp(name, "pair_fill")) ix->opt_pair_fill = value;
-    else if (!strcmp(name, "fused_select")) ix->opt_fused_select = value;
     else if (!strcmp(name, "eval_table")) ix->opt_eval_table = value;
     else if (!strcmp(name, "build_fraction")) ix->opt_build_fraction = value > 0 ? value : 16;
     else if (!strcmp(name, "build_fraction_small")) ix->opt_build_fraction_small = value > 0 ? value : 0;

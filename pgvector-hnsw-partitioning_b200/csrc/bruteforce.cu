@@ -32,7 +32,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdio>
 #include <cstring>
 #include <vector>
 
@@ -53,8 +52,6 @@ struct BfParams {
     float *cand_thr;         // nq x S: score of the K1-th kept row, -inf when the slice kept everything
     float *dbg;              // optional nq x N raw scores (tests)
     float *gthr;             // nq_pad: best K1-th score any finished slice reported for the query (threshold seed)
-    unsigned long long *ev;  // experiments: insertion events, warp-level events
-    int mode;                // experiments: 0 normal, 1 epilogue releases TMEM untouched, 2 epilogue only loads TMEM
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t) __cvta_generic_to_shared(p); }
@@ -235,7 +232,6 @@ bf_gemm_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             // at or below it can never reach the query's top K1 -- skip them from the start
             const float seed = valid_q ? *reinterpret_cast<volatile float *>(p.gthr + q) : NEG_INF;
             float thr = seed;
-            unsigned long long n_ev = 0, n_wev = 0;
             for (int nt = nt0; nt < nt1; nt++) {
                 const int n0 = nt * BF_BN;
                 float *xn = xnh + (nt & 1) * BF_BN;
@@ -248,10 +244,9 @@ bf_gemm_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                 const uint32_t taddr = tmem_base + ((uint32_t) (quarter * 32) << 16) + (uint32_t) acc * BF_BN + half * (BF_BN / 2);
                 const int ncols = min(BF_BN, p.N - n0);       // columns past N are TMA zero fill
 #pragma unroll 1
-                for (int c = 0; c < BF_BN / 64 && p.mode != 1; c++) {
+                for (int c = 0; c < BF_BN / 64; c++) {
                     uint32_t v[32];
                     tmem_ld32(taddr + c * 32, v);
-                    if (p.mode == 2) { if (v[lane] == 0x7fc12345u) ts[0] = 1.f; continue; }
                     const int col0 = half * (BF_BN / 2) + c * 32;
                     if constexpr (DBG) {
                         if (valid_q)
@@ -269,7 +264,6 @@ bf_gemm_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                     float mx = sv[0];
 #pragma unroll
                     for (int i = 1; i < 32; i++) mx = fmaxf(mx, sv[i]);
-                    if (p.mode == 3) n_wev += __any_sync(FULL, valid_q && mx > thr) ? 1 : 0;
                     if (valid_q && mx > thr) {
                         unsigned hits = 0;
 #pragma unroll
@@ -289,7 +283,6 @@ bf_gemm_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                             for (int t = 0; t < 2; t++) m2[t] = (i & 2) ? m4[t + 2] : m4[t];
                             const float sc = (i & 1) ? m2[1] : m2[0];
                             if (!(sc > thr)) continue;                    // the threshold rose inside this chunk
-                            if (p.mode == 3) n_ev++;
                             const int32_t id = n0 + col0 + i;
                             int r0 = 0, r1 = 0, r2 = 0, r3 = 0;           // rank = entries that stay ahead (ties keep earlier columns first)
 #pragma unroll
@@ -317,7 +310,6 @@ bf_gemm_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                 acc ^= 1;
                 if (acc == 0) acc_phase ^= 1;
             }
-            if (p.mode == 3) { atomicAdd(p.ev, n_ev); if (lane == 0) atomicAdd(p.ev + 1, n_wev); }
             if (valid_q) {
                 const size_t slot = (size_t) q * (2 * p.S) + 2 * split + half;
 #pragma unroll
@@ -601,7 +593,6 @@ int hb_bruteforce_ex(hb_index *ix, const void *host_queries, int64_t nq, int k, 
         HB_CK(st.dbg.ensure(sizeof(float) * nq * n));
         p.dbg = st.dbg.as<float>();
     }
-    p.mode = ix->opt_variant;   // experiment knob shared with the scan kernel
     HB_CK(st.gthr.ensure(sizeof(float) * nq_pad));
     {
         std::vector<float> ninf((size_t) nq_pad, -INFINITY);
@@ -609,8 +600,6 @@ int hb_bruteforce_ex(hb_index *ix, const void *host_queries, int64_t nq, int k, 
         HB_CK(cudaStreamSynchronize(s));
     }
     p.gthr = st.gthr.as<float>();
-    p.ev = reinterpret_cast<unsigned long long *>(max_bits + 4);
-    HB_CK(cudaMemsetAsync(p.ev, 0, 16, s));
     CUtensorMap tmA, tmB;
     int rc = make_map(&tmA, st.qb.p, (uint64_t) nq_pad, (uint64_t) kpad, BF_BM);
     if (rc) return rc;
@@ -663,12 +652,6 @@ int hb_bruteforce_ex(hb_index *ix, const void *host_queries, int64_t nq, int k, 
             HB_CK(cudaMemcpyAsync(out_dist + q * k, st.out_dist.as<float>() + q * k, sizeof(float) * k, cudaMemcpyDeviceToHost, s));
         }
         HB_CK(cudaStreamSynchronize(s));
-    }
-    if (p.mode == 3) {
-        unsigned long long ev[2];
-        cudaMemcpy(ev, p.ev, 16, cudaMemcpyDeviceToHost);
-        fprintf(stderr, "[bf] insertion events %llu (%.1f per thread-item), warp-level events %llu, columns per thread-item %d, S=%d\n", ev[0],
-                (double) ev[0] / ((double) nq * 2 * p.S), ev[1], p.tiles_per_split * BF_BN / 2, p.S);
     }
     if (stats) { stats[0] = (float) (nq - n_unc); stats[1] = (float) n_unc; stats[2] = gemm_ms; }
     return HB_OK;

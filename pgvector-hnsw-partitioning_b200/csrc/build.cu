@@ -31,7 +31,6 @@ namespace hb {
 
 #define HB_DECLB(name)                                                                                   \
     cudaError_t build_search_##name(const BuildSearchParams &, int, int, cudaStream_t, bool slow);       \
-    cudaError_t build_select_##name(const BuildSelectParams &, int, cudaStream_t);                       \
     cudaError_t build_link_##name(const LinkParams &, int, int, cudaStream_t);                            \
     cudaError_t pair_fill_##name(const LinkParams &, int, int, cudaStream_t);                           \
     cudaError_t nbr_dist_##name(const NbrDistParams &, int, cudaStream_t);
@@ -377,8 +376,6 @@ int64_t build_insert(hb_index *ix, const void *host_vecs, int64_t n_in, const in
         hb::DevBuf *W = ix->ws_build;
         const int64_t E = b * m2 + UR1 * m;
         HB_CK(W[1].ensure(((size_t) 3 * b + 3 * UR1) * 4 + (size_t) b * 9 + 256));   // packed bookkeeping words
-        HB_CK(W[3].ensure((size_t) b * efc * 8 + sizeof(int32_t) * b));       // cand0 id | d | cnt
-        HB_CK(W[4].ensure((size_t) UR1 * efc * 8 + sizeof(int32_t) * UR1));
         HB_CK(W[5].ensure((size_t) b * m2 * 8 + sizeof(int32_t) * b));        // sel0 id | d | cnt
         HB_CK(W[6].ensure((size_t) UR1 * m * 8 + sizeof(int32_t) * UR1));     // selu id | d | cnt
         HB_CK(W[7].ensure(sizeof(int32_t) * b * DUP_SLOTS));
@@ -617,12 +614,6 @@ int64_t build_insert(hb_index *ix, const void *host_vecs, int64_t n_in, const in
             sp.slots = slots;
             sp.upper_slots = std::min(slots, 1024);
         }
-        sp.cand0_id = W[3].as<int32_t>();
-        sp.cand0_d = reinterpret_cast<float *>(sp.cand0_id + (size_t) b * efc);
-        sp.cand0_cnt = reinterpret_cast<int32_t *>(sp.cand0_d + (size_t) b * efc);
-        sp.candu_id = W[4].as<int32_t>();
-        sp.candu_d = reinterpret_cast<float *>(sp.candu_id + (size_t) UR1 * efc);
-        sp.candu_cnt = reinterpret_cast<int32_t *>(sp.candu_d + (size_t) UR1 * efc);
         sp.status = W[8].as<int32_t>();
         sp.slow_list = sp.status + b;
         sp.slow_count = reinterpret_cast<int32_t *>(misc + 2);
@@ -639,21 +630,14 @@ int64_t build_insert(hb_index *ix, const void *host_vecs, int64_t n_in, const in
         sp.oslots = 4096;
         HB_CK(ix->ws_ovf.ensure(sizeof(uint32_t) * (size_t) ix->num_sms * MAX_CTAS_PER_SM * BUILD_WARPS * sp.oslots));
         sp.ovf = ix->ws_ovf.as<uint32_t>();
-        // ---- neighbour selection: fused into the candidate search unless fused_select = 0
-        BuildSelectParams lp;
-        memset(&lp, 0, sizeof lp);
-        lp.g = sp.g; lp.first = cur; lp.B = (int) b; lp.UR = UR; lp.efc = efc;
-        lp.cand0_id = sp.cand0_id; lp.cand0_d = sp.cand0_d; lp.cand0_cnt = sp.cand0_cnt;
-        lp.candu_id = sp.candu_id; lp.candu_d = sp.candu_d; lp.candu_cnt = sp.candu_cnt;
-        lp.sel0_id = W[5].as<int32_t>();
-        lp.sel0_d = reinterpret_cast<float *>(lp.sel0_id + (size_t) b * m2);
-        lp.sel0_cnt = reinterpret_cast<int32_t *>(lp.sel0_d + (size_t) b * m2);
-        lp.selu_id = W[6].as<int32_t>();
-        lp.selu_d = reinterpret_cast<float *>(lp.selu_id + (size_t) UR1 * m);
-        lp.selu_cnt = reinterpret_cast<int32_t *>(lp.selu_d + (size_t) UR1 * m);
-        lp.dup = W[7].as<int32_t>();
-        lp.totals = ix->d_totals;
-        sp.fuse = ix->opt_fused_select;
+        // ---- neighbour selection, fused into the candidate search: its outputs
+        sp.sel0_id = W[5].as<int32_t>();
+        sp.sel0_d = reinterpret_cast<float *>(sp.sel0_id + (size_t) b * m2);
+        sp.sel0_cnt = reinterpret_cast<int32_t *>(sp.sel0_d + (size_t) b * m2);
+        sp.selu_id = W[6].as<int32_t>();
+        sp.selu_d = reinterpret_cast<float *>(sp.selu_id + (size_t) UR1 * m);
+        sp.selu_cnt = reinterpret_cast<int32_t *>(sp.selu_d + (size_t) UR1 * m);
+        sp.dup = W[7].as<int32_t>();
         uint32_t *et_key = nullptr;
         float *et_val = nullptr;
         if (ix->opt_eval_table) {
@@ -665,8 +649,6 @@ int64_t build_insert(hb_index *ix, const void *host_vecs, int64_t n_in, const in
             sp.el_cap = et_slots / 2;            // a table is at most half full
             HB_CK(cudaMemsetAsync(et_key, 0xff, (size_t) b * et_slots * 4, s));
         }
-        sp.sel0_id = lp.sel0_id; sp.sel0_d = lp.sel0_d; sp.sel0_cnt = lp.sel0_cnt;
-        sp.selu_id = lp.selu_id; sp.selu_d = lp.selu_d; sp.selu_cnt = lp.selu_cnt; sp.dup = lp.dup;
         HB_CK(HB_PICK(build_search, ix)(sp, ix->num_sms, slow_grid, s, false));
         BuildSearchParams sps = sp;
         sps.work = misc + 1; sps.qlist = sp.slow_list; sps.qcount = sp.slow_count;
@@ -678,8 +660,7 @@ int64_t build_insert(hb_index *ix, const void *host_vecs, int64_t n_in, const in
             HB_CK(cudaGetLastError());
         }
         if (trace) cudaEventRecord(tev[1], s);
-        if (!sp.fuse) HB_CK(HB_PICK(build_select, ix)(lp, ix->num_sms, s));
-        build_check_kernel<<<(int) ((b + 255) / 256), 256, 0, s>>>(sp.status, lp.dup, (int) b, d_flag);
+        build_check_kernel<<<(int) ((b + 255) / 256), 256, 0, s>>>(sp.status, sp.dup, (int) b, d_flag);
         HB_CK(cudaGetLastError());
         if (trace) cudaEventRecord(tev[2], s);
 
@@ -709,7 +690,7 @@ int64_t build_insert(hb_index *ix, const void *host_vecs, int64_t n_in, const in
             CommitParams cp;
             cp.B = (int) b; cp.UR = UR; cp.m = m;
             cp.final_id = d_final; cp.new_uoff = d_nuoff; cp.tid = d_tid; cp.dest_urow = d_durow;
-            cp.sel0_id = lp.sel0_id; cp.sel0_d = lp.sel0_d; cp.selu_id = lp.selu_id; cp.selu_d = lp.selu_d;
+            cp.sel0_id = sp.sel0_id; cp.sel0_d = sp.sel0_d; cp.selu_id = sp.selu_id; cp.selu_d = sp.selu_d;
             cp.nbr0 = ix->d_nbr0; cp.nbr0d = ix->d_nbr0d; cp.nbru = ix->d_nbru; cp.nbrud = ix->d_nbrud;
             cp.uoff = ix->d_uoff; cp.tid0 = ix->d_tid0; cp.ntids = ix->d_ntids;
             cp.pv0 = ix->d_pv0; cp.pvu = ix->d_pvu;
@@ -720,8 +701,8 @@ int64_t build_insert(hb_index *ix, const void *host_vecs, int64_t n_in, const in
             EdgeGenParams gp;
             gp.B = (int) b; gp.UR = UR; gp.m = m; gp.first = cur;
             gp.final_id = d_final; gp.urow_owner = d_uown; gp.urow_layer = d_ulay;
-            gp.sel0_id = lp.sel0_id; gp.sel0_d = lp.sel0_d; gp.sel0_cnt = lp.sel0_cnt;
-            gp.selu_id = lp.selu_id; gp.selu_d = lp.selu_d; gp.selu_cnt = lp.selu_cnt;
+            gp.sel0_id = sp.sel0_id; gp.sel0_d = sp.sel0_d; gp.sel0_cnt = sp.sel0_cnt;
+            gp.selu_id = sp.selu_id; gp.selu_d = sp.selu_d; gp.selu_cnt = sp.selu_cnt;
             gp.key = key_in; gp.val = val_in; gp.flag = d_flag;
             edge_gen_kernel<<<tgrid, 256, 0, s>>>(gp);
             HB_CK(cudaGetLastError());
@@ -783,7 +764,7 @@ int64_t build_insert(hb_index *ix, const void *host_vecs, int64_t n_in, const in
         if (flag & 2) {
             // FindDuplicateInMemory: fold a tuple into the first byte-identical neighbour with room
             dup.resize((size_t) b * DUP_SLOTS);
-            HB_CK(cudaMemcpyAsync(dup.data(), lp.dup, sizeof(int32_t) * b * DUP_SLOTS, cudaMemcpyDeviceToHost, s));
+            HB_CK(cudaMemcpyAsync(dup.data(), sp.dup, sizeof(int32_t) * b * DUP_SLOTS, cudaMemcpyDeviceToHost, s));
             HB_CK(cudaStreamSynchronize(s));
             next = cur;
             urows = ix->upper_rows;

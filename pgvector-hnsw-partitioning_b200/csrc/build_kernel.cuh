@@ -6,7 +6,6 @@
 //                            SelectNeighbors + CheckElementCloser (heuristic with pruned back-fill) and
 //                            hnswbuild.c FindDuplicateInMemory, for a whole batch of new elements against
 //                            the graph as it stood before the batch
-//   build_select_kernel   <- the selection as a kernel of its own (fused_select = 0)
 //   build_commit_kernel   <- hnswutils.c AddConnections (build.cu)
 //   link_memo_kernel /    <- hnswutils.c HnswUpdateConnection (reverse links; re-selection when the
 //   link_pipe_kernel /       neighbour's list is full), one warp or CTA per (target, layer), edges
@@ -33,8 +32,6 @@ struct BuildSearchParams {
     const uint8_t *level;        // B
     const int32_t *ucand_row;    // B: first upper candidate row of element i (layers 1..), or -1
     int efc, slots, upper_slots, capW;
-    int32_t *cand0_id; float *cand0_d; int32_t *cand0_cnt;   // B x efc, nearest first
-    int32_t *candu_id; float *candu_d; int32_t *candu_cnt;   // UR x efc
     int32_t *status, *slow_list, *slow_count;
     const int32_t *qlist, *qcount;
     unsigned long long *totals;
@@ -42,13 +39,12 @@ struct BuildSearchParams {
     uint32_t *ovf; int oslots;    // fast path: per-warp visited overflow table in HBM
     uint32_t *gbits; int gwords;
     float *gwd; uint32_t *gwi; int gcap;
-    // fused selection (fuse != 0): SelectNeighbors runs on each layer's W as soon as that layer's
-    // search is done -- the selection work of finished elements fills the tail of the batch's search
-    // -- and the candidate lists are not written out
-    int fuse;
+    // SelectNeighbors runs on each layer's W as soon as that layer's search is done -- the selection
+    // work of finished elements fills the tail of the batch's search -- so the candidate lists are
+    // never written out
     int32_t *sel0_id; float *sel0_d; int32_t *sel0_cnt;     // B x 2m
     int32_t *selu_id; float *selu_d; int32_t *selu_cnt;     // UR x m
-    int32_t *dup;                                           // B x DUP_SLOTS
+    int32_t *dup;                                           // B x DUP_SLOTS: leading byte-identical neighbours
     // evaluated-distance logs (search_core.cuh EvalLog), B x el_cap entries each + B counts; NULL = not kept
     uint32_t *el_id; float *el_d; int32_t *el_n; int el_cap;
 };
@@ -150,54 +146,41 @@ __global__ void __launch_bounds__(BUILD_WARPS * 32, (NV == 1 ? 6 : 4)) build_sea
             if (st != ST_OK) break;
             keep = p.efc;
             const int cnt = min(w.L, p.efc);
-            if (p.fuse) {
-                // SelectNeighbors on this layer's candidates (W is only read: it is the next layer's entry list)
-                const int lm = lc == 0 ? lm0 : g.m;
-                const size_t row = lc == 0 ? (size_t) i : (size_t) p.ucand_row[i] + (lc - 1);
-                __syncwarp();
-                for (int j = lane; j < cnt; j += 32) c_id[j] = (int32_t) (w.id[j] & ID_MASK);
-                __syncwarp();
-                int32_t pruned;
-                const int nr = select_neighbors_warp<T, IP, NV, (G > 4 ? 4 : G)>(g, q, c_id, w.d, cnt, lm, r_id, r_d, wd_id, wd_d, pruned,
-                                                                                lane, np_e);
-                int32_t *oid = (lc == 0 ? p.sel0_id : p.selu_id) + row * lm;
-                float *od = (lc == 0 ? p.sel0_d : p.selu_d) + row * lm;
-                for (int j = lane; j < lm; j += 32) { oid[j] = j < nr ? r_id[j] : -1; od[j] = j < nr ? r_d[j] : 0.f; }
-                if (lane == 0) (lc == 0 ? p.sel0_cnt : p.selu_cnt)[row] = nr;
-                if (lc == 0) {
-                    // FindDuplicateInMemory: neighbours in stored order while byte-identical to the new row
-                    const uint4 *mine = reinterpret_cast<const uint4 *>(g.vecs + (size_t) (p.first + i) * g.row_bytes);
-                    int nd = 0;
-                    for (int j = 0; j < nr && nd < DUP_SLOTS; j++) {
-                        const uint4 *other = reinterpret_cast<const uint4 *>(g.vecs + (size_t) r_id[j] * g.row_bytes);
-                        bool same = true;
-                        for (int ch = lane; ch < g.nvec; ch += 32) {
-                            const uint4 a = mine[ch], b = other[ch];
-                            same = same && a.x == b.x && a.y == b.y && a.z == b.z && a.w == b.w;
-                        }
-                        if (!__all_sync(FULL, same)) break;
-                        if (lane == 0) p.dup[(size_t) i * DUP_SLOTS + nd] = r_id[j];
-                        nd++;
-                    }
-                    if (lane == 0 && nd < DUP_SLOTS) p.dup[(size_t) i * DUP_SLOTS + nd] = -1;
-                } else {
-                    // the selection staged candidate rows over the query: put the query back for the next layer
-                    __syncwarp();
-                    stage_row<T>(g.vecs + (size_t) (p.first + i) * g.row_bytes, g.nvec, q, lane);
-                    __syncwarp();
-                }
-                continue;
-            }
-            int32_t *cid; float *cd;
+            // SelectNeighbors on this layer's candidates (W is only read: it is the next layer's entry list)
+            const int lm = lc == 0 ? lm0 : g.m;
+            const size_t row = lc == 0 ? (size_t) i : (size_t) p.ucand_row[i] + (lc - 1);
+            __syncwarp();
+            for (int j = lane; j < cnt; j += 32) c_id[j] = (int32_t) (w.id[j] & ID_MASK);
+            __syncwarp();
+            int32_t pruned;
+            const int nr = select_neighbors_warp<T, IP, NV, (G > 4 ? 4 : G)>(g, q, c_id, w.d, cnt, lm, r_id, r_d, wd_id, wd_d, pruned,
+                                                                            lane, np_e);
+            int32_t *oid = (lc == 0 ? p.sel0_id : p.selu_id) + row * lm;
+            float *od = (lc == 0 ? p.sel0_d : p.selu_d) + row * lm;
+            for (int j = lane; j < lm; j += 32) { oid[j] = j < nr ? r_id[j] : -1; od[j] = j < nr ? r_d[j] : 0.f; }
+            if (lane == 0) (lc == 0 ? p.sel0_cnt : p.selu_cnt)[row] = nr;
             if (lc == 0) {
-                cid = p.cand0_id + (size_t) i * p.efc; cd = p.cand0_d + (size_t) i * p.efc;
-                if (lane == 0) p.cand0_cnt[i] = cnt;
+                // FindDuplicateInMemory: neighbours in stored order while byte-identical to the new row
+                const uint4 *mine = reinterpret_cast<const uint4 *>(g.vecs + (size_t) (p.first + i) * g.row_bytes);
+                int nd = 0;
+                for (int j = 0; j < nr && nd < DUP_SLOTS; j++) {
+                    const uint4 *other = reinterpret_cast<const uint4 *>(g.vecs + (size_t) r_id[j] * g.row_bytes);
+                    bool same = true;
+                    for (int ch = lane; ch < g.nvec; ch += 32) {
+                        const uint4 a = mine[ch], b = other[ch];
+                        same = same && a.x == b.x && a.y == b.y && a.z == b.z && a.w == b.w;
+                    }
+                    if (!__all_sync(FULL, same)) break;
+                    if (lane == 0) p.dup[(size_t) i * DUP_SLOTS + nd] = r_id[j];
+                    nd++;
+                }
+                if (lane == 0 && nd < DUP_SLOTS) p.dup[(size_t) i * DUP_SLOTS + nd] = -1;
             } else {
-                const size_t row = (size_t) p.ucand_row[i] + (lc - 1);
-                cid = p.candu_id + row * p.efc; cd = p.candu_d + row * p.efc;
-                if (lane == 0) p.candu_cnt[row] = cnt;
+                // the selection staged candidate rows over the query: put the query back for the next layer
+                __syncwarp();
+                stage_row<T>(g.vecs + (size_t) (p.first + i) * g.row_bytes, g.nvec, q, lane);
+                __syncwarp();
             }
-            for (int j = lane; j < cnt; j += 32) { cid[j] = (int32_t) (w.id[j] & ID_MASK); cd[j] = w.d[j]; }
         }
         if (st != ST_OK && !SLOW) {
             if (lane == 0) {
@@ -276,77 +259,10 @@ __device__ __forceinline__ int select_neighbors_warp(const GraphView &g, float *
     return nr;
 }
 
-struct BuildSelectParams {
-    GraphView g;
-    int64_t first;
-    int B, UR, efc;
-    const int32_t *cand0_id; const float *cand0_d; const int32_t *cand0_cnt;
-    const int32_t *candu_id; const float *candu_d; const int32_t *candu_cnt;
-    int32_t *sel0_id; float *sel0_d; int32_t *sel0_cnt;     // B x 2m
-    int32_t *selu_id; float *selu_d; int32_t *selu_cnt;     // UR x m
-    int32_t *dup;                                           // B x DUP_SLOTS: leading byte-identical neighbours
-    unsigned long long *totals;
-};
-
 template <typename T> __host__ __device__ inline size_t select_warp_smem(int nvec, int nc_max, int lm_max)
 {
     size_t b = (size_t) nvec * Vec<T>::VEC * 4 + (size_t) nc_max * 16 + (size_t) lm_max * 8;
     return (b + 15) & ~(size_t) 15;
-}
-
-template <typename T, int IP, int NV, int G>
-__global__ void __launch_bounds__(BUILD_WARPS * 32) build_select_kernel(const BuildSelectParams p)
-{
-    extern __shared__ __align__(16) unsigned char smem[];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const GraphView &g = p.g;
-    const int lm0 = 2 * g.m;
-    unsigned char *base = smem + select_warp_smem<T>(g.nvec, p.efc, lm0) * warp;
-    float *q = reinterpret_cast<float *>(base);
-    int32_t *c_id = reinterpret_cast<int32_t *>(base + (size_t) g.nvec * Vec<T>::VEC * 4);
-    float *c_d = reinterpret_cast<float *>(c_id + p.efc);
-    int32_t *wd_id = reinterpret_cast<int32_t *>(c_d + p.efc);
-    float *wd_d = reinterpret_cast<float *>(wd_id + p.efc);
-    int32_t *r_id = reinterpret_cast<int32_t *>(wd_d + p.efc);
-    float *r_d = reinterpret_cast<float *>(r_id + lm0);
-
-    const int items = p.B + p.UR;
-    unsigned long long npair = 0;
-    for (int item = blockIdx.x * BUILD_WARPS + warp; item < items; item += gridDim.x * BUILD_WARPS) {
-        const bool base_layer = item < p.B;
-        const int row = base_layer ? item : item - p.B;
-        const int nc = base_layer ? p.cand0_cnt[row] : p.candu_cnt[row];
-        const int32_t *gid = (base_layer ? p.cand0_id : p.candu_id) + (size_t) row * p.efc;
-        const float *gd = (base_layer ? p.cand0_d : p.candu_d) + (size_t) row * p.efc;
-        const int lm = base_layer ? lm0 : g.m;
-        __syncwarp();
-        for (int j = lane; j < nc; j += 32) { c_id[j] = gid[j]; c_d[j] = gd[j]; }
-        __syncwarp();
-        int32_t pruned;
-        const int nr = select_neighbors_warp<T, IP, NV, G>(g, q, c_id, c_d, nc, lm, r_id, r_d, wd_id, wd_d, pruned, lane, npair);
-        int32_t *oid = (base_layer ? p.sel0_id : p.selu_id) + (size_t) row * lm;
-        float *od = (base_layer ? p.sel0_d : p.selu_d) + (size_t) row * lm;
-        for (int j = lane; j < lm; j += 32) { oid[j] = j < nr ? r_id[j] : -1; od[j] = j < nr ? r_d[j] : 0.f; }
-        if (lane == 0) (base_layer ? p.sel0_cnt : p.selu_cnt)[row] = nr;
-        if (base_layer) {
-            // FindDuplicateInMemory: neighbours in stored order while byte-identical to the new row
-            const uint4 *mine = reinterpret_cast<const uint4 *>(g.vecs + (size_t) (p.first + row) * g.row_bytes);
-            int nd = 0;
-            for (int j = 0; j < nr && nd < DUP_SLOTS; j++) {
-                const uint4 *other = reinterpret_cast<const uint4 *>(g.vecs + (size_t) r_id[j] * g.row_bytes);
-                bool same = true;
-                for (int ch = lane; ch < g.nvec; ch += 32) {
-                    const uint4 a = mine[ch], b = other[ch];
-                    same = same && a.x == b.x && a.y == b.y && a.z == b.z && a.w == b.w;
-                }
-                if (!__all_sync(FULL, same)) break;
-                if (lane == 0) p.dup[(size_t) row * DUP_SLOTS + nd] = r_id[j];
-                nd++;
-            }
-            if (lane == 0 && nd < DUP_SLOTS) p.dup[(size_t) row * DUP_SLOTS + nd] = -1;
-        }
-    }
-    if (lane == 0 && npair) atomicAdd(p.totals + 4, npair);
 }
 
 // ---- HnswUpdateConnection, one warp per segment (see link_kernel.cuh) --------------------------
@@ -751,29 +667,6 @@ cudaError_t launch_build_search_t(const BuildSearchParams &p, int num_sms, int s
                     err = cudaGetLastError();                                                      \
                 }                                                                                  \
             }                                                                                      \
-        }                                                                                          \
-    }
-    HB_NV_DISPATCH(p.g.nvec, HB_CALL)
-#undef HB_CALL
-    return err;
-}
-
-template <typename T, int IP>
-cudaError_t launch_build_select_t(const BuildSelectParams &p, int num_sms, cudaStream_t stream)
-{
-    cudaError_t err = cudaSuccess;
-    const int items = p.B + p.UR;
-    if (items <= 0) return err;
-#define HB_CALL(NVV, GG)                                                                           \
-    {                                                                                              \
-        auto kern = build_select_kernel<T, IP, NVV, (GG > 4 ? 4 : GG)>;                            \
-        const size_t smem = select_warp_smem<T>(p.g.nvec, p.efc, 2 * p.g.m) * BUILD_WARPS;         \
-        err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem); \
-        if (err == cudaSuccess) {                                                                  \
-            int grid = (items + BUILD_WARPS - 1) / BUILD_WARPS;                                    \
-            if (grid > num_sms * 8) grid = num_sms * 8;                                            \
-            kern<<<grid, BUILD_WARPS * 32, smem, stream>>>(p);                                     \
-            err = cudaGetLastError();                                                              \
         }                                                                                          \
     }
     HB_NV_DISPATCH(p.g.nvec, HB_CALL)

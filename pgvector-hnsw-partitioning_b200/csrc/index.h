@@ -101,8 +101,9 @@ struct hb_index {
     std::vector<uint8_t> h_deleted;   // HnswElementTupleData.deleted: set by hb_vacuum_repair's MarkDeleted (may be shorter than n)
 
     // tuning knobs (0 = automatic)
-    int opt_slots = 0, opt_grid = 0, opt_build_batch = 0, opt_per_query = 0, opt_variant = 0, opt_no_slow = 0;
-    int opt_pair_cache = 1, opt_pair_fill = 1, opt_fused_select = 1, opt_eval_table = 1;
+    int opt_slots = 0, opt_grid = 0, opt_build_batch = 0, opt_per_query = 0;
+    int opt_variant = 0;           // the scan path forced for tests (ScanVariant, scan_kernel.cuh)
+    int opt_pair_cache = 1, opt_pair_fill = 1, opt_eval_table = 1;
     int opt_auto_grow = 1;         // inserts beyond the capacity grow the index (hb_index_reserve) instead of failing
     int opt_build_fraction = 16;   // a batch is at most 1/opt_build_fraction of the graph
     int opt_build_fraction_small = 0;    // the same while the graph holds fewer than 65536 elements (the latency-bound start-up); 0 = automatic

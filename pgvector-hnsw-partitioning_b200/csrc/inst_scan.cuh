@@ -32,10 +32,6 @@ cudaError_t HB_CAT(build_search_, HBI_NAME)(const BuildSearchParams &p, int sms,
     return slow ? launch_build_search_t<HBI_T, HBI_IP, true>(p, sms, slow_grid, s)
                 : launch_build_search_t<HBI_T, HBI_IP, false>(p, sms, slow_grid, s);
 }
-cudaError_t HB_CAT(build_select_, HBI_NAME)(const BuildSelectParams &p, int sms, cudaStream_t s)
-{
-    return launch_build_select_t<HBI_T, HBI_IP>(p, sms, s);
-}
 cudaError_t HB_CAT(build_link_, HBI_NAME)(const LinkParams &p, int sms, int which, cudaStream_t s)
 {
     return launch_build_link_t<HBI_T, HBI_IP>(p, sms, which, s);

@@ -526,7 +526,6 @@ hb_part *hb_part_create(int device, int dim, int m, int ef_construction, int met
     // all-gather's and the merges' CTAs must not queue behind a whole batch of them
     int prio_lo = 0, prio_hi = 0;
     if (cudaSetDevice(device) == cudaSuccess) cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
-    if (const char *e = getenv("HB_PART_XS_PRIORITY")) { if (atoi(e) == 0) prio_hi = prio_lo; }      // experiments: 0 = default priority
     if (cudaSetDevice(device) != cudaSuccess || cudaStreamCreateWithPriority(&pt->xs, cudaStreamNonBlocking, prio_hi) != cudaSuccess) {
         set_error("hb_part_create: no CUDA device %d; there is no CPU fallback", device);
         hb_part_free(pt);
@@ -537,7 +536,6 @@ hb_part *hb_part_create(int device, int dim, int m, int ef_construction, int met
         hb_part_free(pt);
         return nullptr;
     }
-    if (const char *e = getenv("HB_PART_EXCHANGE")) pt->exchange = atoi(e);                          // experiments: 0 = ncclAllGather
     if (world > PART_MAX_WORLD) pt->exchange = 0;
     if (world > 1) {
         NcclApi *nc = nccl_api();

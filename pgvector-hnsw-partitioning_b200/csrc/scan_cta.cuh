@@ -570,10 +570,9 @@ cudaError_t launch_scan_cta_variant(const ScanParams &p, int num_sms, cudaStream
     int dev = 0;
     cudaGetDevice(&dev);
     dev &= 15;
-    const int sub = p.variant / 10;                   // experiments: 1 = list in shared memory, 2 = no row staging
-    if (sub != 1 && p.ef + 24 <= 128 && p.out_stride <= 128) {
+    if (p.variant != SCAN_CTA_SMEM_LIST && p.ef + 24 <= 128 && p.out_stride <= 128) {
         auto kern = scan_cta_reg_kernel<T, IP, NV, 4>;
-        const bool stage = sub != 2 && 2 * p.g.m <= 32 && scan_cta_reg_smem<T>(p.g.nvec, p.g.row_bytes, true) <= 200 * 1024;
+        const bool stage = p.variant != SCAN_CTA_NO_STAGE && 2 * p.g.m <= 32 && scan_cta_reg_smem<T>(p.g.nvec, p.g.row_bytes, true) <= 200 * 1024;
         const size_t smem = scan_cta_reg_smem<T>(p.g.nvec, p.g.row_bytes, stage);
         static thread_local size_t seen_reg[16];
         if (seen_reg[dev] < smem) {
@@ -599,11 +598,11 @@ cudaError_t launch_scan_cta_variant(const ScanParams &p, int num_sms, cudaStream
 // batches small enough that the GPU is mostly idle: one CTA per query (shared memory must hold the list and the table)
 inline bool use_cta_scan(const ScanParams &p, int num_sms, size_t row_smem_bytes, const void *ep, int variant)
 {
-    if (ep != nullptr || variant == 9 || variant == 6) return false;
+    if (ep != nullptr || variant == SCAN_SMEM_LIST || variant == SCAN_NO_CTA) return false;
     if (p.nq > num_sms) return false;
-    const bool forced = variant % 10 == 7;
+    const bool forced = variant == SCAN_CTA || variant == SCAN_CTA_SMEM_LIST || variant == SCAN_CTA_NO_STAGE;
     // measured (profiles/r2_experiments.md): rows of 3 KB gain 15-20 % at 32..148 queries; rows of 512 B lose 15-25 %
-    // to the register-list kernel, whose hop is shorter than this kernel's three block barriers.  variant 7 forces it.
+    // to the register-list kernel, whose hop is shorter than this kernel's three block barriers.  SCAN_CTA forces it.
     if (p.g.nvec < 96 && !forced) return false;
     return row_smem_bytes + (size_t) p.capW * 8 + (size_t) CTA_SLOTS * 4 + 1024 <= 200 * 1024;
 }

@@ -14,6 +14,22 @@ namespace hb {
 constexpr int SCAN_WARPS = 4;   // warps (= concurrent queries) per CTA
 constexpr int MAX_CTAS_PER_SM = 12;   // cap on resident CTAs per SM (sizes the per-warp overflow tables)
 
+// hb_set_option("variant"): the scan path forced for tests, so that every production kernel can be checked against
+// the others on any shape.  All of them give identical results.
+enum ScanVariant {
+    SCAN_AUTO = 0,
+    SCAN_NO_CTA = 6,            // never the CTA-per-query kernels of small batches (scan_cta.cuh)
+    SCAN_CTA = 7,               // the CTA-per-query kernels for every row length, in the form the shape selects
+    SCAN_SMEM_LIST = 9,         // the shared-memory-list warp kernel instead of the register-list one, no CTA kernels
+    SCAN_CTA_SMEM_LIST = 17,    // as SCAN_CTA, with the list in shared memory
+    SCAN_CTA_NO_STAGE = 27,     // as SCAN_CTA, the register list without row staging
+};
+inline bool is_scan_variant(int v)
+{
+    return v == SCAN_AUTO || v == SCAN_NO_CTA || v == SCAN_CTA || v == SCAN_SMEM_LIST || v == SCAN_CTA_SMEM_LIST ||
+           v == SCAN_CTA_NO_STAGE;
+}
+
 struct ScanParams {
     GraphView g;
     const void *queries;       // nq x dim, index dtype, already normalised when cosine
@@ -38,7 +54,7 @@ struct ScanParams {
     float *gwd; uint32_t *gwi; int gcap;
     // single-layer mode (unit tests): explicit entry points
     const int32_t *ep; int nep; int layer;
-    int variant;               // host only: tuning variant of the unrolled kernel (0 = default)
+    int variant;               // host only: the forced scan path (ScanVariant)
 };
 
 template <typename T> __host__ __device__ inline size_t scan_warp_smem(int nvec, int capW, int slots, bool slow)
@@ -48,11 +64,11 @@ template <typename T> __host__ __device__ inline size_t scan_warp_smem(int nvec,
     return (b + 15) & ~(size_t) 15;
 }
 
-// WPB warps (= concurrent queries) per CTA.  SCAN_WARPS here: with rows of several kB one-warp CTAs measured 12 % slower
+// SCAN_WARPS warps (= concurrent queries) per CTA: with rows of several kB one-warp CTAs measured 12 % slower
 // (3.56 vs 4.05 M queries/s at 1M x 768 in the same run), while the register-list kernel for short rows gains 5-9 % from
 // them (profiles/r2_experiments.md).
-template <typename T, int IP, int NV, int G, bool SLOW, int MINB, int WPB = SCAN_WARPS>
-__global__ void __launch_bounds__(WPB * 32, MINB * (SCAN_WARPS / WPB)) scan_kernel(const ScanParams p)
+template <typename T, int IP, int NV, int G, bool SLOW, int MINB>
+__global__ void __launch_bounds__(SCAN_WARPS * 32, MINB) scan_kernel(const ScanParams p)
 {
     extern __shared__ __align__(16) unsigned char smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -65,7 +81,7 @@ __global__ void __launch_bounds__(WPB * 32, MINB * (SCAN_WARPS / WPB)) scan_kern
     WList w;
     VS vs;
     if constexpr (SLOW) {
-        const size_t gw = (size_t) blockIdx.x * WPB + warp;
+        const size_t gw = (size_t) blockIdx.x * SCAN_WARPS + warp;
         vs.bits = p.gbits + gw * p.gwords;
         vs.words = p.gwords;
         w.d = p.gwd + gw * p.gcap;
@@ -74,7 +90,7 @@ __global__ void __launch_bounds__(WPB * 32, MINB * (SCAN_WARPS / WPB)) scan_kern
     } else {
         unsigned char *s = base + (size_t) g.nvec * Vec<T>::VEC * 4;
         vs.tab = reinterpret_cast<uint32_t *>(s);
-        vs.set_overflow(p.ovf + ((size_t) blockIdx.x * WPB + warp) * p.oslots, p.oslots);
+        vs.set_overflow(p.ovf + ((size_t) blockIdx.x * SCAN_WARPS + warp) * p.oslots, p.oslots);
         w.d = reinterpret_cast<float *>(s + (size_t) p.slots * 4);
         w.id = reinterpret_cast<uint32_t *>(s + (size_t) p.slots * 4 + (size_t) p.capW * 4);
         w.cap = p.capW;
@@ -165,12 +181,13 @@ __global__ void __launch_bounds__(WPB * 32, MINB * (SCAN_WARPS / WPB)) scan_kern
 // host-side launch helper -------------------------------------------------------------------
 struct ScanLaunchInfo { int grid; size_t smem; int blocks_per_sm; };
 
-template <typename T, int IP, int NV, int G, bool SLOW, int MINB, int WPB = SCAN_WARPS>
-cudaError_t launch_scan_variant(const ScanParams &p, int num_sms, int max_grid, cudaStream_t stream,
-                                ScanLaunchInfo *info)
+// Persistent CTAs of WARPS warps that pull queries from p.work: as many CTAs as are resident, no more than `want` and,
+// when max_grid > 0, no more than max_grid.  The kernel is a template argument so that each kernel caches its own
+// occupancy.
+template <void (*KERN)(ScanParams), int WARPS>
+cudaError_t launch_persistent(const ScanParams &p, size_t smem, int64_t want, int num_sms, int max_grid, cudaStream_t stream,
+                              ScanLaunchInfo *info)
 {
-    auto kern = scan_kernel<T, IP, NV, G, SLOW, MINB, WPB>;
-    const size_t smem = scan_warp_smem<T>(p.g.nvec, p.capW, p.slots, SLOW) * WPB;
     // the function attribute and the occupancy query cost several microseconds each: remember them per
     // device for the shared-memory size last used (a single scan is only ~350 us long); per host thread,
     // so that handles driven from different threads never share mutable state
@@ -182,20 +199,19 @@ cudaError_t launch_scan_variant(const ScanParams &p, int num_sms, int max_grid, 
     int bps = 0;
     if (seen_bps[dev] > 0 && seen_smem[dev] == smem) bps = seen_bps[dev];
     else {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
+        cudaError_t e = cudaFuncSetAttribute(KERN, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
         if (e != cudaSuccess) return e;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kern, WPB * 32, smem);
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, KERN, WARPS * 32, smem);
         if (e != cudaSuccess) return e;
         if (bps < 1) return cudaErrorInvalidConfiguration;
         seen_smem[dev] = smem; seen_bps[dev] = bps;
     }
-    if (bps * WPB > MAX_CTAS_PER_SM * SCAN_WARPS) bps = MAX_CTAS_PER_SM * SCAN_WARPS / WPB;     // the overflow tables are sized for this many warps
-    int64_t want = SLOW ? max_grid : (p.nq + WPB - 1) / WPB;
+    if (bps * WARPS > MAX_CTAS_PER_SM * SCAN_WARPS) bps = MAX_CTAS_PER_SM * SCAN_WARPS / WARPS;     // the overflow tables are sized for this many warps
     int grid = (int) (want < (int64_t) bps * num_sms ? want : (int64_t) bps * num_sms);
     if (max_grid > 0 && grid > max_grid) grid = max_grid;
     if (grid < 1) grid = 1;
     if (info) { info->grid = grid; info->smem = smem; info->blocks_per_sm = bps; }
-    kern<<<grid, WPB * 32, smem, stream>>>(p);
+    KERN<<<grid, WARPS * 32, smem, stream>>>(p);
     return cudaGetLastError();
 }
 
@@ -213,34 +229,19 @@ template <typename T, int IP, bool SLOW>
 cudaError_t launch_scan_t(const ScanParams &p, int num_sms, int max_grid, cudaStream_t stream,
                           ScanLaunchInfo *info)
 {
-    if constexpr (SLOW) return launch_scan_variant<T, IP, 0, 2, true, 1>(p, num_sms, max_grid, stream, info);
+    const size_t smem = scan_warp_smem<T>(p.g.nvec, p.capW, p.slots, SLOW) * SCAN_WARPS;
+    const int64_t want = SLOW ? max_grid : (p.nq + SCAN_WARPS - 1) / SCAN_WARPS;
+#define HB_LAUNCH(NVV, GG, MB) launch_persistent<scan_kernel<T, IP, NVV, GG, SLOW, MB>, SCAN_WARPS>(p, smem, want, num_sms, max_grid, stream, info)
+    if constexpr (SLOW) return HB_LAUNCH(0, 2, 1);
     else {
-        if (nv_of(p.g.nvec) == 6 && p.variant) {
-            switch (p.variant) {
-            case 8: return launch_scan_variant<T, IP, 6, 4, false, 4, 1>(p, num_sms, max_grid, stream, info);      // one warp per CTA
-            case 1: return launch_scan_variant<T, IP, 6, 4, false, 3>(p, num_sms, max_grid, stream, info);
-            case 2: return launch_scan_variant<T, IP, 6, 2, false, 4>(p, num_sms, max_grid, stream, info);
-            case 3: return launch_scan_variant<T, IP, 6, 2, false, 5>(p, num_sms, max_grid, stream, info);
-            case 4: return launch_scan_variant<T, IP, 6, 2, false, 6>(p, num_sms, max_grid, stream, info);
-            case 5: return launch_scan_variant<T, IP, 6, 1, false, 6>(p, num_sms, max_grid, stream, info);
-            default: break;
-            }
-        }
-        if (nv_of(p.g.nvec) == 1 && p.variant) {
-            switch (p.variant) {
-            case 1: return launch_scan_variant<T, IP, 1, 8, false, 8>(p, num_sms, max_grid, stream, info);
-            case 2: return launch_scan_variant<T, IP, 1, 4, false, 8>(p, num_sms, max_grid, stream, info);
-            case 3: return launch_scan_variant<T, IP, 1, 8, false, 5>(p, num_sms, max_grid, stream, info);
-            default: break;
-            }
-        }
         switch (nv_of(p.g.nvec)) {
-#define HB_CASE(NVV, GG, MB) case NVV: return launch_scan_variant<T, IP, NVV, GG, false, MB>(p, num_sms, max_grid, stream, info);
+#define HB_CASE(NVV, GG, MB) case NVV: return HB_LAUNCH(NVV, GG, MB);
             HB_NV_TABLE(HB_CASE)
 #undef HB_CASE
-        default: return launch_scan_variant<T, IP, 0, 2, false, 4>(p, num_sms, max_grid, stream, info);
+        default: return HB_LAUNCH(0, 2, 4);
         }
     }
+#undef HB_LAUNCH
 }
 
 // ---- the query-vs-neighbour-list distance kernel on its own (opclass FUNCTION 1, batched) ----

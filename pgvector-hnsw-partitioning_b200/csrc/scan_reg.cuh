@@ -293,11 +293,13 @@ template <typename T> __host__ __device__ inline size_t scan_reg_warp_smem(int n
     return (((size_t) nvec * Vec<T>::VEC * 4 + (size_t) slots * 4 + 128) + 15) & ~(size_t) 15;
 }
 
-// WPB warps (= concurrent queries) per CTA.  One warp per CTA by default: a CTA's resources come back the moment its
-// last query is done, so the tail of one batch overlaps the start of the next at warp granularity (with four warps per
-// CTA three idle warps wait for the straggler; measured in profiles/r2_experiments.md).
-template <typename T, int IP, int NV, int G, int R, int MINB, int WPB>
-__global__ void __launch_bounds__(WPB * 32, MINB) scan_reg_kernel(const ScanParams p)
+// One warp (= one concurrent query) per CTA: a CTA's resources come back the moment its last query is done, so the tail
+// of one batch overlaps the start of the next at warp granularity (with four warps per CTA three idle warps wait for the
+// straggler; measured in profiles/r2_experiments.md).
+constexpr int SCAN_REG_WARPS = 1;
+
+template <typename T, int IP, int NV, int G, int R, int MINB>
+__global__ void __launch_bounds__(SCAN_REG_WARPS * 32, MINB) scan_reg_kernel(const ScanParams p)
 {
     extern __shared__ __align__(16) unsigned char smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -307,7 +309,7 @@ __global__ void __launch_bounds__(WPB * 32, MINB) scan_reg_kernel(const ScanPara
     int32_t *cbuf = reinterpret_cast<int32_t *>(base + (size_t) g.nvec * Vec<T>::VEC * 4);
     VisitedHash vs;
     vs.tab = reinterpret_cast<uint32_t *>(cbuf + 32);
-    vs.set_overflow(p.ovf + ((size_t) blockIdx.x * WPB + warp) * p.oslots, p.oslots);
+    vs.set_overflow(p.ovf + ((size_t) blockIdx.x * SCAN_REG_WARPS + warp) * p.oslots, p.oslots);
     RegW<R> w;
     const int ef = p.ef;
 
@@ -374,41 +376,11 @@ __global__ void __launch_bounds__(WPB * 32, MINB) scan_reg_kernel(const ScanPara
     }
 }
 
-template <typename T, int IP, int NV, int G, int R, int MINB, int WPB>
-cudaError_t launch_scan_reg_variant(const ScanParams &p, int num_sms, int max_grid, cudaStream_t stream, ScanLaunchInfo *info)
-{
-    auto kern = scan_reg_kernel<T, IP, NV, G, R, MINB, WPB>;
-    const size_t smem = scan_reg_warp_smem<T>(p.g.nvec, p.slots) * WPB;
-    static thread_local size_t seen_smem[16];
-    static thread_local int seen_bps[16];
-    int dev = 0;
-    cudaGetDevice(&dev);
-    dev &= 15;
-    int bps = 0;
-    if (seen_bps[dev] > 0 && seen_smem[dev] == smem) bps = seen_bps[dev];
-    else {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
-        if (e != cudaSuccess) return e;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kern, WPB * 32, smem);
-        if (e != cudaSuccess) return e;
-        if (bps < 1) return cudaErrorInvalidConfiguration;
-        seen_smem[dev] = smem; seen_bps[dev] = bps;
-    }
-    if (bps * WPB > MAX_CTAS_PER_SM * SCAN_WARPS) bps = MAX_CTAS_PER_SM * SCAN_WARPS / WPB;     // the overflow tables are sized for this many warps
-    const int64_t want = (p.nq + WPB - 1) / WPB;
-    int grid = (int) (want < (int64_t) bps * num_sms ? want : (int64_t) bps * num_sms);
-    if (max_grid > 0 && grid > max_grid) grid = max_grid;
-    if (grid < 1) grid = 1;
-    if (info) { info->grid = grid; info->smem = smem; info->blocks_per_sm = bps; }
-    kern<<<grid, WPB * 32, smem, stream>>>(p);
-    return cudaGetLastError();
-}
-
 // rows short enough that bookkeeping, not bytes, bounds the scan (one or two 128-bit loads per lane): the
 // register-list kernel when the list fits (ef + room for the tie tail <= 32 R)
 inline int reg_list_R(int nvec, int ef, const void *ep, int variant)
 {
-    if (ep != nullptr || variant == 9) return 0;           // single-layer test surface / forced shared-memory list
+    if (ep != nullptr || variant == SCAN_SMEM_LIST) return 0;      // single-layer test surface / forced shared-memory list
     const int nv = nv_of(nvec);
     if (nv != 1 && nv != 2) return 0;
     if (ef + 16 <= 64) return 2;
@@ -419,19 +391,15 @@ inline int reg_list_R(int nvec, int ef, const void *ep, int variant)
 template <typename T, int IP>
 cudaError_t launch_scan_reg_t(const ScanParams &p, int R, int num_sms, int max_grid, cudaStream_t stream, ScanLaunchInfo *info)
 {
+    const size_t smem = scan_reg_warp_smem<T>(p.g.nvec, p.slots) * SCAN_REG_WARPS;
+    const int64_t want = (p.nq + SCAN_REG_WARPS - 1) / SCAN_REG_WARPS;
     const int nv = nv_of(p.g.nvec);
-    if (nv == 1 && R == 2 && p.variant) {       // experiments (hb_set_option "variant"): four warps per CTA, other occupancies
-        switch (p.variant) {
-        case 1: return launch_scan_reg_variant<T, IP, 1, 8, 2, 6, 4>(p, num_sms, max_grid, stream, info);
-        case 2: return launch_scan_reg_variant<T, IP, 1, 4, 2, 32, 1>(p, num_sms, max_grid, stream, info);
-        case 3: return launch_scan_reg_variant<T, IP, 1, 8, 2, 8, 4>(p, num_sms, max_grid, stream, info);
-        default: break;
-        }
-    }
-    if (nv == 1 && R == 2) return launch_scan_reg_variant<T, IP, 1, 8, 2, 24, 1>(p, num_sms, max_grid, stream, info);
-    if (nv == 1 && R == 4) return launch_scan_reg_variant<T, IP, 1, 8, 4, 24, 1>(p, num_sms, max_grid, stream, info);
-    if (nv == 2 && R == 2) return launch_scan_reg_variant<T, IP, 2, 8, 2, 16, 1>(p, num_sms, max_grid, stream, info);
-    if (nv == 2 && R == 4) return launch_scan_reg_variant<T, IP, 2, 8, 4, 16, 1>(p, num_sms, max_grid, stream, info);
+#define HB_LAUNCH(NVV, RR, MB) launch_persistent<scan_reg_kernel<T, IP, NVV, 8, RR, MB>, SCAN_REG_WARPS>(p, smem, want, num_sms, max_grid, stream, info)
+    if (nv == 1 && R == 2) return HB_LAUNCH(1, 2, 24);
+    if (nv == 1 && R == 4) return HB_LAUNCH(1, 4, 24);
+    if (nv == 2 && R == 2) return HB_LAUNCH(2, 2, 16);
+    if (nv == 2 && R == 4) return HB_LAUNCH(2, 4, 16);
+#undef HB_LAUNCH
     return cudaErrorInvalidConfiguration;
 }
 

@@ -409,3 +409,17 @@ def test_cta_per_query_tie_tail(oracle, pkg):
         check_scan(oracle, orc, ix, q, 48, natural_check=False)
         check_scan(oracle, orc, ix, q, 10, natural_check=False)
     ix.close()
+
+
+def test_scan_variant_values(pkg):
+    """The variant option takes only the values that force a production scan path; the removed tuning variants and
+    the unfused neighbour selection are refused instead of silently ignored."""
+    ix = pkg.HnswIndex(128, "vector_l2_ops", 16, 64, capacity=10)
+    for v in (1, 2, 3, 4, 5, 8, 10, 20):
+        with pytest.raises(pkg.HnswError):
+            ix.set_option("variant", v)
+    for v in (0, 6, 7, 9, 17, 27):
+        ix.set_option("variant", v)
+    with pytest.raises(pkg.HnswError):
+        ix.set_option("fused_select", 0)
+    ix.close()

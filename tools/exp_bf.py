@@ -19,7 +19,6 @@ g.uoff, g.nbru, g.ntids, g.tids = np.full(n, -1, np.int32), np.full((1, 16), -1,
 ix.load_graph(g)
 q = gen_set(nq, dim, 20260102 + 1000, dev)
 qh = q.cpu().numpy()
-ix.set_option("variant", int(os.environ.get("BFMODE", "0")))
 for it in range(3):
     t0 = time.time()
     elem, dist, st = ix.bruteforce(qh, 10, stats=True)

@@ -1,6 +1,6 @@
 """Scan-kernel experiment driver: build an index of a given shape on the GPU, then time the batched scan for a
 list of (variant, streams) settings.  Used for A/B runs and as the ncu target for the scan kernels.
-usage: python tools/exp_scan.py --rows 1000000 --dim 128 --ef 40 [--opclass vector_l2_ops] [--variants 0,1,2]
+usage: python tools/exp_scan.py --rows 1000000 --dim 128 --ef 40 [--opclass vector_l2_ops] [--variants 0,6,9]
                                 [--streams 1,3] [--steps 10] [--nq 10000] [--latency]"""
 import argparse
 import os
