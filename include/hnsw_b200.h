@@ -108,7 +108,9 @@ int hb_index_trim(hb_index *ix);
 int hb_set_build_batch(hb_index *ix, int max_batch);
 /* HnswInitElement's level draw for the seq-th initialised element: (int)(-ln(U) / ln(m)), capped */
 int hb_level_for(uint64_t seed, int64_t seq, int m);
-/* tuning knobs: "slots" (visited-table size), "grid" (CTA cap), "build_batch",
+/* tuning knobs: "slots" (visited-table size), "grid" (CTA cap of the persistent scans and of the exact scan;
+ * the exact scan splits its work the same way under any cap, so a cap only makes each CTA run more work items and
+ * the answer does not change), "build_batch",
  * "per_query_counters" (0/1), "variant" (scan kernel forced for tests: 0 automatic; 6 never the
  * four-warps-per-query kernels of small batches; 7 / 17 / 27 those kernels for every row length: default form /
  * list in shared memory / no row staging; 9 the shared-memory-list warp kernel instead of the register-list one;
@@ -234,7 +236,9 @@ int hb_bruteforce(hb_index *ix, const void *host_queries, int64_t nq, int k, int
                   float *out_dist);
 /* same, with diagnostics: dbg_scores (optional, host, nq x n) receives the raw bf16 GEMM scores;
  * stats (optional, 3 floats): queries certified exact by the bf16 error bound, queries re-scanned
- * exhaustively in fp32, GEMM kernel milliseconds.  1 <= k <= 128. */
+ * exhaustively in fp32, GEMM kernel milliseconds.  1 <= k <= 128.  Either way the answer is the exact top-k
+ * of the canonical fp32 distance (FUNCTION 1) by (distance, element id), padded with -1 / +inf when n < k.
+ * hb_set_option(ix, "grid", g) caps the GEMM kernel's CTAs at g. */
 int hb_bruteforce_ex(hb_index *ix, const void *host_queries, int64_t nq, int k, int32_t *out_elem,
                      float *out_dist, float *dbg_scores, float *stats);
 

@@ -1133,6 +1133,33 @@ void orc_bruteforce(const OrcIndex *ix, const void *queries, int64_t nq, int k, 
     }
 }
 
+void orc_exact_topk(const OrcIndex *ix, const void *queries, int64_t nq, int k, int32_t *out_elem,
+                    float *out_dist, int threads)
+{
+    int dim = ix->dim;
+    size_t rowb = (size_t) dim * ix->esize;
+    if (threads < 1) threads = 1;
+#pragma omp parallel for num_threads(threads) schedule(dynamic, 4)
+    for (int64_t qi = 0; qi < nq; qi++) {
+        float q[dim];
+        query_as_float(ix, (const char *) queries + (size_t) qi * rowb, q);
+        Cand *top = malloc(sizeof(Cand) * (size_t) k);
+        int nt = 0;
+        for (int64_t e = 0; e < ix->n; e++) {
+            Cand c = { dist_q_row(ix, q, row_of(ix, e)), (int32_t) e };
+            if (nt == k && !key_lt(c, top[k - 1])) continue;
+            int p = nt < k ? nt++ : k - 1;
+            while (p > 0 && key_lt(c, top[p - 1])) { top[p] = top[p - 1]; p--; }
+            top[p] = c;
+        }
+        for (int j = 0; j < k; j++) {
+            out_elem[qi * k + j] = j < nt ? top[j].id : -1;
+            out_dist[qi * k + j] = j < nt ? top[j].d : INFINITY;
+        }
+        free(top);
+    }
+}
+
 /* ------------------------------------------------------------------ flat image */
 
 int64_t orc_n(const OrcIndex *ix) { return ix->n; }

@@ -98,6 +98,11 @@ int orc_search_layer(const OrcIndex *ix, const void *query, const int32_t *ep, i
  * (normalised for cosine) vectors; ties by element id. out: nq x k. */
 void orc_bruteforce(const OrcIndex *ix, const void *queries, int64_t nq, int k, int32_t *out_elem,
                     double *out_dist, int threads);
+/* exact top-k in the library's own arithmetic (the exact scan's contract): every row's canonical fp32
+ * FUNCTION 1 distance (dist_q_row; cosine queries normalised as by the scans), the k smallest by
+ * (distance, element id), padded with -1 / +inf when n < k.  out: nq x k. */
+void orc_exact_topk(const OrcIndex *ix, const void *queries, int64_t nq, int k, int32_t *out_elem,
+                    float *out_dist, int threads);
 
 /* scalar entry points (vector.c / halfutils.c support functions); metric_is_ip: 0 = squared l2,
  * 1 = negative inner product, ORC_L1 = l1 */

@@ -72,6 +72,7 @@ def lib():
     L.orc_search_layer.restype = C.c_int
     L.orc_search_layer.argtypes = [C.c_void_p, vp, i32p, C.c_int, C.c_int, C.c_int, i32p, f32p, C.POINTER(Counters)]
     L.orc_bruteforce.argtypes = [C.c_void_p, vp, C.c_int64, C.c_int, i32p, vp, C.c_int]
+    L.orc_exact_topk.argtypes = [C.c_void_p, vp, C.c_int64, C.c_int, i32p, f32p, C.c_int]
     L.orc_iter_begin.restype = C.c_void_p
     L.orc_iter_begin.argtypes = [C.c_void_p, vp, C.c_int, C.c_int64]
     L.orc_iter_next.restype = C.c_int
@@ -254,6 +255,15 @@ class Index:
         e = np.empty((nq, k), np.int32)
         d = np.empty((nq, k), np.float64)
         lib().orc_bruteforce(self._h, _p(qs), nq, k, _p(e), _p(d), threads)
+        return e, d
+
+    def exact_topk(self, qs, k, threads=1):
+        """top-k by the canonical fp32 distance and element id over every row (the exact scan's answer)"""
+        qs = self._q(qs)
+        nq = qs.shape[0]
+        e = np.empty((nq, k), np.int32)
+        d = np.empty((nq, k), np.float32)
+        lib().orc_exact_topk(self._h, _p(qs), nq, k, _p(e), _p(d), threads)
         return e, d
 
     def export(self):

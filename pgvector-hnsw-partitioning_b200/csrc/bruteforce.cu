@@ -12,10 +12,10 @@
 //      slices of the same query that already finished (global per-query K1-th score), which cuts the
 //      insertions ~4x.
 //   2. fp32 re-rank: the exact canonical-order distance (distance.cuh) of every candidate.
-//   3. certification: bf16 rounding perturbs a dot product by at most (2^-8 + 2^-11)*|q|*|x|, so any
-//      row that was NOT kept has a true distance above a bound computed from the slice threshold; if
-//      that bound exceeds the k-th exact distance the result is provably the exact top-k.  Queries
-//      that cannot be certified are re-scanned exhaustively in fp32.
+//   3. certification: bf16 rounding, the GEMM's fp32 accumulation and the fp32 norms perturb a score by
+//      a bounded amount (bf_select_kernel), so any row that was NOT kept has a canonical distance above a
+//      bound computed from the slice threshold; if that bound exceeds the k-th exact distance the result
+//      is provably the exact top-k.  Queries that cannot be certified are re-scanned exhaustively in fp32.
 //
 // Warp roles (320 threads, one CTA per SM, persistent over (query tile, X slice) work items ordered
 // slice-major so the CTAs of a wave stream the same rows of X through L2 together):
@@ -234,7 +234,12 @@ bf_gemm_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             float thr = seed;
             for (int nt = nt0; nt < nt1; nt++) {
                 const int n0 = nt * BF_BN;
-                float *xn = xnh + (nt & 1) * BF_BN;
+                // chosen by the accumulator index, not by nt: acc flips on every tile of the CTA's life, also from
+                // one work item to the next.  A warp that finished tile t stages tile t+1 into the other buffer;
+                // it can reach this buffer again only for tile t+2, after every epilogue warp passed tile t+1's
+                // barrier, i.e. finished reading tile t.  (nt's parity repeats across two items of one CTA when
+                // tiles_per_split is odd.)
+                float *xn = xnh + acc * BF_BN;
                 if constexpr (L2) {
                     for (int c = et; c < BF_BN; c += 32 * BF_EPI_WARPS) xn[c] = (n0 + c) < p.N ? p.xnh[n0 + c] : 0.f;
                     asm volatile("bar.sync 1, %0;" ::"n"(32 * BF_EPI_WARPS) : "memory");
@@ -325,33 +330,73 @@ bf_gemm_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     }
 }
 
-// rows of the index (padded fp32 / fp16 rows) -> bf16 [n x kpad], plus 0.5|x|^2 and max |x|
+// rows of the index (padded fp32 / fp16 rows) -> bf16 [n x kpad], plus per row 0.5|x|^2 (xnh) and the squared norm
+// of the bf16 rounding error |bf16(x) - x|^2 (err2), and/or the maxima of both over the rows (maxes[0], maxes[1]:
+// fp32 bits, non-negative, so they order as unsigned integers).  Each is an fp32 sum of kpad/32 lane-strided
+// terms and a 5-level butterfly: relative error at most gamma(kpad/32 + 6) (bf_select_kernel).
 template <typename T>
 __global__ void to_bf16_kernel(const char *__restrict__ rows, size_t row_bytes, int dim, int kpad, int64_t n,
-                               __nv_bfloat16 *__restrict__ out, float *__restrict__ xnh, unsigned int *__restrict__ max_norm_bits)
+                               __nv_bfloat16 *__restrict__ out, float *__restrict__ xnh, float *__restrict__ err2,
+                               unsigned int *__restrict__ maxes)
 {
     const int lane = threadIdx.x & 31;
     const int64_t r = (int64_t) blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (r >= n) return;
     const T *src = reinterpret_cast<const T *>(rows + r * row_bytes);
-    float s = 0.f;
+    float s = 0.f, e2 = 0.f;
     for (int e = lane; e < kpad; e += 32) {
         const float v = e < dim ? (float) src[e] : 0.f;
+        const __nv_bfloat16 b = __float2bfloat16_rn(v);
+        const float d = __bfloat162float(b) - v;      // exact: the low bits the rounding dropped
         s += v * v;
-        out[r * kpad + e] = __float2bfloat16_rn(v);
+        e2 += d * d;
+        out[r * kpad + e] = b;
     }
-    for (int b = 16; b >= 1; b >>= 1) s += __shfl_xor_sync(FULL, s, b);
+    for (int b = 16; b >= 1; b >>= 1) {
+        s += __shfl_xor_sync(FULL, s, b);
+        e2 += __shfl_xor_sync(FULL, e2, b);
+    }
     if (lane == 0) {
         if (xnh) xnh[r] = 0.5f * s;
-        if (max_norm_bits) atomicMax(max_norm_bits, __float_as_uint(sqrtf(s) * 1.000001f));
+        if (err2) err2[r] = e2;
+        if (maxes) {
+            atomicMax(maxes, __float_as_uint(0.5f * s));
+            atomicMax(maxes + 1, __float_as_uint(e2));
+        }
     }
 }
 
-// exact fp32 re-rank results -> top-k by (distance, id) and the certificate
+__device__ __forceinline__ double gamma_fp32(double m) { return m * 0x1p-24 / (1.0 - m * 0x1p-24); }
+
+// exact fp32 re-rank results -> top-k by (distance, id) and the certificate.
+//
+// Certificate.  Every row a slice did not keep has GEMM score s <= thr (thr: the slice's cut-off, seeds included).
+// Take q the exact-path query (normalised for cosine), x a row, ^ their bf16 copies, u = 2^-24,
+// gamma(m) = m u / (1 - m u).  The score differs from the exact q.x (inner product, cosine) or q.x - |x|^2/2 (L2)
+// by at most
+//   E = |q^ - q| |x^| + |q| |x^ - x|                       bf16 rounding of both operands ((q^-q).x^ + q.(x^-x))
+//     + g_acc |q^| |x^|,  g_acc = kpad 2^-23 / (1 - kpad 2^-23)     the GEMM's fp32 accumulation over kpad terms, in
+//                                                          any order and with truncating adds (2^-23, not 2^-24)
+//   L2 only:
+//     + g_h H                                              |x|^2/2 as to_bf16_kernel sums it
+//     + u (|q^| |x^| (1 + g_acc) + H)                      the rounding of score = acc - |x|^2/2
+// with |x^| <= X + D, |q^| <= |q| + |q^ - q|, X = max |x|, D = max |x^ - x|, H = max |x|^2/2 over the rows.  Every
+// norm is the fp32 sum of to_bf16_kernel widened by its own error, g_h = gamma(kpad/32 + 6).  So a dropped row has
+//   inner product / cosine:  q.x <= thr + E
+//   L2:                      |q - x|^2 = |q|^2 - 2 (q.x - |x|^2/2) >= |q|^2 - 2 (thr + E)
+// and its canonical fp32 distance (the re-rank's, distance.cuh: FMA chains of at most kpad/32 terms, <= 3 folds, a
+// 5-level butterfly, so depth m_c <= kpad/32 + 8) is at least
+//   inner product / cosine:  -(thr + E) - gamma(m_c) |q| X
+//   L2:                      (|q|^2 - 2 (thr + E)) (1 - gamma(m_c + 2))    (+2: q_i - x_i is rounded before squaring)
+// This bound lb is evaluated in double; 2^-40 of its magnitude covers that evaluation's own rounding.  When
+// lb > tau, the k-th re-ranked fp32 distance, for every slice, no dropped row can enter the top-k, not even on an id
+// tie, and the answer is the exact one; otherwise the query is re-scanned in fp32.  The terms scale with |q||x| and
+// with |x|^2: a query at the origin keeps the |x|^2 terms, which is what rows of almost equal norm need.
 __global__ void bf_select_kernel(const int32_t *__restrict__ cand_id, const float *__restrict__ cand_dist,
                                  const float *__restrict__ cand_thr, const float *__restrict__ qnorm2h,
-                                 const unsigned int *__restrict__ max_norm_bits, int nq, int S, int k, int l2,
-                                 int32_t *__restrict__ out_elem, float *__restrict__ out_dist, int32_t *__restrict__ uncertain)
+                                 const float *__restrict__ qerr2, const unsigned int *__restrict__ maxes, int nq, int S,
+                                 int k, int kpad, int l2, int32_t *__restrict__ out_elem, float *__restrict__ out_dist,
+                                 int32_t *__restrict__ uncertain)
 {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= nq) return;
@@ -372,17 +417,23 @@ __global__ void bf_select_kernel(const int32_t *__restrict__ cand_id, const floa
         out_elem[(size_t) q * k + j] = j < cnt ? bi[j] : -1;
         out_dist[(size_t) q * k + j] = j < cnt ? bd[j] : __int_as_float(0x7f800000);
     }
-    // certificate: every row a slice did not keep has bf16 score <= thr, so its true score is at most
-    // thr + E with E = (2^-8 + 2^-11) |q| |x|max
-    const float qn = sqrtf(2.f * qnorm2h[q]);
-    const float E = (1.f / 256.f + 1.f / 2048.f) * qn * __uint_as_float(*max_norm_bits);
     bool ok = true;
     if (cnt == k) {
-        const float tau = bd[k - 1];
+        const double g_h = gamma_fp32(kpad / 32 + 6), g_c = gamma_fp32(kpad / 32 + 8);
+        const double g_acc = kpad * 0x1p-23 / (1.0 - kpad * 0x1p-23);
+        const double q2hi = 2.0 * qnorm2h[q] / (1.0 - g_h), q2lo = 2.0 * qnorm2h[q] / (1.0 + g_h);   // |q|^2
+        const double Q = sqrt(q2hi), Qe = sqrt((double) qerr2[q] / (1.0 - g_h));
+        const double H = __uint_as_float(maxes[0]) / (1.0 - g_h);
+        const double X = sqrt(2.0 * H), D = sqrt((double) __uint_as_float(maxes[1]) / (1.0 - g_h));
+        const double QX = (Q + Qe) * (X + D);                                                   // |q^| |x^|
+        double E = Qe * (X + D) + Q * D + g_acc * QX;
+        if (l2) E += g_h * H + 0x1p-24 * (QX * (1.0 + g_acc) + H);
+        const double tau = bd[k - 1];
         for (int s = 0; s < S && ok; s++) {
             const float thr = cand_thr[(size_t) q * S + s];
             if (thr == __int_as_float(0xff800000)) continue;
-            const float lb = l2 ? (2.f * qnorm2h[q] - 2.f * (thr + E)) : -(thr + E);
+            double lb = l2 ? (q2lo - 2.0 * (thr + E)) * (1.0 - gamma_fp32(kpad / 32 + 10)) : -(thr + E) - g_c * Q * X;
+            lb -= 0x1p-40 * (fabs((double) thr) + E + q2hi + Q * X);
             ok = lb > tau;
         }
     } else {
@@ -469,7 +520,7 @@ static int make_map(CUtensorMap *map, void *base, uint64_t rows, uint64_t kpad, 
 }
 
 struct BfState {
-    DevBuf gthr, xb, xnh, misc, qraw, qn, qb, qnh, cand_score, cand_id, cand_thr, cand_dist, out_elem, out_dist, uncertain, iota, full_dist, dbg;
+    DevBuf gthr, xb, xnh, misc, qraw, qn, qb, qnh, qe, cand_score, cand_id, cand_thr, cand_dist, out_elem, out_dist, uncertain, iota, full_dist, dbg;
     int64_t built_n = -1;
     uint64_t built_gen = 0;      // hb_index::generation the bf16 image was made from
     int kpad = 0;
@@ -487,7 +538,7 @@ void bruteforce_release(hb_index *ix)
     if (!ix->bf) return;
     BfState *s = static_cast<BfState *>(ix->bf);
     ix->bf = nullptr;
-    DevBuf *b[] = { &s->gthr, &s->xb, &s->xnh, &s->misc, &s->qraw, &s->qn, &s->qb, &s->qnh, &s->cand_score, &s->cand_id, &s->cand_thr,
+    DevBuf *b[] = { &s->gthr, &s->xb, &s->xnh, &s->misc, &s->qraw, &s->qn, &s->qb, &s->qnh, &s->qe, &s->cand_score, &s->cand_id, &s->cand_thr,
                     &s->cand_dist, &s->out_elem, &s->out_dist, &s->uncertain, &s->iota, &s->full_dist, &s->dbg };
     for (auto x : b) x->release();
     delete s;
@@ -522,18 +573,18 @@ int hb_bruteforce_ex(hb_index *ix, const void *host_queries, int64_t nq, int k, 
     const int kpad = ((ix->dim + BF_BK - 1) / BF_BK) * BF_BK;
     const bool l2 = ix->metric == HB_L2;
     HB_CK(st.misc.ensure(64));
-    unsigned int *max_bits = st.misc.as<unsigned int>();
+    unsigned int *row_max = st.misc.as<unsigned int>();     // [0] max |x|^2/2, [1] max |bf16(x) - x|^2 (fp32 bits)
 
     // bf16 image of the partition (rebuilt whenever the index changed: every mutation bumps the generation)
     if (st.built_n != n || st.kpad != kpad || st.built_gen != ix->generation) {
         HB_CK(st.xb.ensure((size_t) n * kpad * 2));
         HB_CK(st.xnh.ensure(sizeof(float) * n));
-        HB_CK(cudaMemsetAsync(max_bits, 0, 4, s));
+        HB_CK(cudaMemsetAsync(row_max, 0, 2 * sizeof(unsigned int), s));
         const int wpb = 8, grid = (int) ((n + wpb - 1) / wpb);
         if (ix->dtype == HB_F32)
-            to_bf16_kernel<float><<<grid, wpb * 32, 0, s>>>(ix->d_vecs, ix->row_bytes, ix->dim, kpad, n, st.xb.as<__nv_bfloat16>(), st.xnh.as<float>(), max_bits);
+            to_bf16_kernel<float><<<grid, wpb * 32, 0, s>>>(ix->d_vecs, ix->row_bytes, ix->dim, kpad, n, st.xb.as<__nv_bfloat16>(), st.xnh.as<float>(), nullptr, row_max);
         else
-            to_bf16_kernel<__half><<<grid, wpb * 32, 0, s>>>(ix->d_vecs, ix->row_bytes, ix->dim, kpad, n, st.xb.as<__nv_bfloat16>(), st.xnh.as<float>(), max_bits);
+            to_bf16_kernel<__half><<<grid, wpb * 32, 0, s>>>(ix->d_vecs, ix->row_bytes, ix->dim, kpad, n, st.xb.as<__nv_bfloat16>(), st.xnh.as<float>(), nullptr, row_max);
         HB_CK(cudaGetLastError());
         st.built_n = n; st.kpad = kpad; st.built_gen = ix->generation;
     }
@@ -546,6 +597,7 @@ int hb_bruteforce_ex(hb_index *ix, const void *host_queries, int64_t nq, int k, 
     HB_CK(st.qn.ensure(qbytes));
     HB_CK(st.qb.ensure((size_t) nq_pad * kpad * 2));
     HB_CK(st.qnh.ensure(sizeof(float) * nq_pad));
+    HB_CK(st.qe.ensure(sizeof(float) * nq_pad));
     HB_CK(cudaMemcpyAsync(st.qraw.p, host_queries, qbytes, cudaMemcpyHostToDevice, s));
     const void *qexact = st.qraw.p;
     if (ix->metric == HB_COSINE) {
@@ -558,9 +610,9 @@ int hb_bruteforce_ex(hb_index *ix, const void *host_queries, int64_t nq, int k, 
         const int wpb = 8, grid = (int) ((nq + wpb - 1) / wpb);
         const size_t qrow = (size_t) ix->dim * ix->esize;
         if (ix->dtype == HB_F32)
-            to_bf16_kernel<float><<<grid, wpb * 32, 0, s>>>((const char *) qexact, qrow, ix->dim, kpad, nq, st.qb.as<__nv_bfloat16>(), st.qnh.as<float>(), nullptr);
+            to_bf16_kernel<float><<<grid, wpb * 32, 0, s>>>((const char *) qexact, qrow, ix->dim, kpad, nq, st.qb.as<__nv_bfloat16>(), st.qnh.as<float>(), st.qe.as<float>(), nullptr);
         else
-            to_bf16_kernel<__half><<<grid, wpb * 32, 0, s>>>((const char *) qexact, qrow, ix->dim, kpad, nq, st.qb.as<__nv_bfloat16>(), st.qnh.as<float>(), nullptr);
+            to_bf16_kernel<__half><<<grid, wpb * 32, 0, s>>>((const char *) qexact, qrow, ix->dim, kpad, nq, st.qb.as<__nv_bfloat16>(), st.qnh.as<float>(), st.qe.as<float>(), nullptr);
         HB_CK(cudaGetLastError());
     }
 
@@ -606,7 +658,9 @@ int hb_bruteforce_ex(hb_index *ix, const void *host_queries, int64_t nq, int k, 
     rc = make_map(&tmB, st.xb.p, (uint64_t) n, (uint64_t) kpad, BF_BN);
     if (rc) return rc;
     const int items = p.n_mtiles * p.S;
-    const int grid = std::min(items, ix->num_sms);
+    // the "grid" option caps the CTAs: each then runs more work items; S above depends on num_sms only, so the
+    // answer does not change
+    const int grid = std::min(items, ix->opt_grid > 0 ? std::min(ix->opt_grid, ix->num_sms) : ix->num_sms);
     auto kern = dbg_scores ? (l2 ? bf_gemm_topk_kernel<true, true> : bf_gemm_topk_kernel<true, false>)
                            : (l2 ? bf_gemm_topk_kernel<false, true> : bf_gemm_topk_kernel<false, false>);
     HB_CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) BF_SMEM));
@@ -620,7 +674,7 @@ int hb_bruteforce_ex(hb_index *ix, const void *host_queries, int64_t nq, int k, 
     dp.g = ix->view(); dp.queries = qexact; dp.nq = nq; dp.cand = st.cand_id.as<int32_t>(); dp.nc = (int) C; dp.out = st.cand_dist.as<float>();
     HB_CK(get_dist_launcher(ix->dtype, metric_kind(ix->metric))(dp, s));
     bf_select_kernel<<<(int) ((nq + 63) / 64), 64, 0, s>>>(st.cand_id.as<int32_t>(), st.cand_dist.as<float>(), st.cand_thr.as<float>(),
-                                                          st.qnh.as<float>(), max_bits, (int) nq, S2, k, l2 ? 1 : 0,
+                                                          st.qnh.as<float>(), st.qe.as<float>(), row_max, (int) nq, S2, k, kpad, l2 ? 1 : 0,
                                                           st.out_elem.as<int32_t>(), st.out_dist.as<float>(), st.uncertain.as<int32_t>());
     HB_CK(cudaGetLastError());
     std::vector<int32_t> unc(nq);
