@@ -259,7 +259,11 @@ int hb_elements_to_tids_dev(hb_index *ix, const int32_t *dev_elem, const float *
 /* One process per GPU.  A row belongs to partition splitmix64(heap_tid) mod P; rank r owns the partitions
  * {p : p mod world == r}, each an ordinary hb_index on the rank's GPU.  A search sends the same query batch
  * to every partition, merges the owned partitions' top-k on the device, exchanges the per-rank lists (12 bytes
- * per result) and merges again: every rank ends with the same nq x k answer, ordered by (distance, heap TID).
+ * per result) and merges again: every rank ends with the same nq x k answer.  For each query that answer is the
+ * k smallest (distance, heap TID) pairs over every heap TID of the elements each partition's scan returned (at
+ * most ef_search per partition, each TID at its element's distance), nearest first, ties by heap TID, padded
+ * with -1 / +inf.  It depends neither on the order a scan emits TIDs in (hb_search_batch and hb_gettuple keep
+ * pgvector's gettuple order: an element's TIDs last to first) nor on how partitions are grouped into ranks.
  * The exchange is an all-gather done with stores into the peers' memory over NVLink (buffers mapped through CUDA
  * IPC, epoch flags instead of a collective kernel) or, with hb_part_set_option("exchange", 0) or when peer mapping
  * is not possible, ONE ncclAllGather.  The handle owns the NCCL communicator (NCCL is dlopen'ed when world > 1);

@@ -7,7 +7,7 @@
 //
 // Data path of one search batch on a rank (nothing returns to the host in between):
 //   queries (already on every rank, or ncclBroadcast from the root rank)
-//     -> one scan per owned partition (hb_search_batch_dev + TID mapping), on the slot's sub-streams
+//     -> one scan per owned partition (hb_search_batch_dev + part_tids_kernel), on the slot's sub-streams
 //     -> part_merge_kernel over the owned partitions' lists -> packed block [tids nq x k | dist nq x k]
 //     -> ONE ncclAllGather of that block (12 bytes per result)      -- the only exchange
 //     -> part_merge_kernel over the world's blocks -> result, identical on every rank.
@@ -82,11 +82,58 @@ static NcclApi *nccl_api()
         }                                                                                                 \
     } while (0)
 
+// ---- one partition's list -------------------------------------------------------------------
+// The partitioned answer of a query is the k smallest (distance, heap TID) pairs over every heap TID of the elements
+// the partitions' scans returned.  This kernel writes one partition's share of it: the scan's elements (elem / dist:
+// nq x ef, nearest-first, -1 padded) expanded to all their heap TIDs at the element's distance, the k smallest pairs
+// kept sorted by (distance, tid) in the partition's list block, padded with -1 / +inf.  hnswgettuple's emission order
+// (elements_to_tids_kernel: an element's TIDs last to first) would let the fold of duplicates into elements and the
+// order of TIDs within an element decide which tied TIDs survive; this key does not.  One thread per query.  The
+// elements come in non-decreasing distance, so a new pair only moves past kept pairs of equal distance, and once k
+// are kept the first element beyond the k-th distance ends the walk.  Elements without heap TIDs (deleted, not yet
+// vacuumed) contribute nothing.
+__global__ void part_tids_kernel(const int32_t *__restrict__ elem, const float *__restrict__ dist, int64_t nq, int ef,
+                                 int k, const int64_t *__restrict__ tid0, const uint8_t *__restrict__ ntids,
+                                 const int64_t *__restrict__ tidx, int64_t *__restrict__ out_tids,
+                                 float *__restrict__ out_dist)
+{
+    const int64_t qi = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+    if (qi >= nq) return;
+    int64_t *ot = out_tids + qi * k;
+    float *od = out_dist + qi * k;
+    int o = 0;
+    for (int j = 0; j < ef; j++) {
+        const int32_t e = elem[qi * ef + j];
+        if (e < 0) break;
+        const float d = dist[qi * ef + j];
+        if (o == k && d > od[k - 1]) break;
+        const int nt = ntids[e];
+        for (int t = 0; t < nt; t++) {
+            const int64_t tid = t == 0 ? tid0[e] : tidx[(int64_t) e * (HB_HEAPTIDS - 1) + (t - 1)];
+            int i;
+            if (o < k) i = o++;
+            else if (d < od[k - 1] || (d == od[k - 1] && tid < ot[k - 1])) i = k - 1;
+            else continue;
+            for (; i > 0 && (od[i - 1] > d || (od[i - 1] == d && ot[i - 1] > tid)); i--) {
+                ot[i] = ot[i - 1];
+                od[i] = od[i - 1];
+            }
+            ot[i] = tid;
+            od[i] = d;
+        }
+    }
+    for (; o < k; o++) {
+        ot[o] = -1;
+        od[o] = __int_as_float(0x7f800000);
+    }
+}
+
 // ---- merge ----------------------------------------------------------------------------------
-// A "block" is one list set for nq queries: [tids nq x k int64 | dist nq x k fp32], nearest-first, padded with
-// tid -1 / +inf.  Greedy head merge of n_lists blocks (block l at base + l * stride bytes) ordered by
-// (distance, tid): since the key is a total order the result does not depend on how the lists are grouped
-// (merging per rank and then across ranks equals one flat merge over all partitions).
+// A "block" is one list set for nq queries: [tids nq x k int64 | dist nq x k fp32], sorted by (distance, tid), padded
+// with tid -1 / +inf.  Greedy head merge of n_lists blocks (block l at base + l * stride bytes) ordered by
+// (distance, tid): the inputs are sorted by that key, so the output is the k smallest pairs of their union, and since
+// the key is a total order the result does not depend on how the lists are grouped (merging per rank and then across
+// ranks equals one flat merge over all partitions).
 __global__ void part_merge_kernel(const char *__restrict__ base, int n_lists, size_t stride, int64_t nq, int k,
                                   char *__restrict__ out)
 {
@@ -726,8 +773,9 @@ int hb_part_search_async(hb_part *pt, int slot, const void *queries, int queries
         int32_t *cnt = S.cnt.as<int32_t>() + (size_t) i * nq;
         rc = hb_search_batch_dev(ix, dq, nq, ef_search, elem, edist, cnt, (void *) t);
         if (rc) return rc;
-        rc = hb_elements_to_tids_dev(ix, elem, edist, nq, ef_search, k, l_tids, l_dist, (void *) t);
-        if (rc) return rc;
+        part_tids_kernel<<<(int) ((nq + 127) / 128), 128, 0, t>>>(elem, edist, nq, ef_search, k, ix->d_tid0, ix->d_ntids,
+                                                                   ix->d_tidx, l_tids, l_dist);
+        HB_CK(cudaGetLastError());
         auto it = ix->stream_ws.find((void *) t);
         if (it != ix->stream_ws.end()) {
             part_status_kernel<<<1, 1, 0, t>>>(it->second->misc.as<int32_t>() + 3, S.status.as<int32_t>());

@@ -31,9 +31,10 @@ def split_rows(heap_tids, n_partitions, rank, world):
 
 
 def merge_rule(lists, k):
-    """The merge contract of part_merge_kernel restated for tests: greedy head merge of per-partition lists
-    [(tids, dist), ...] (each nearest-first, -1 padded) ordered by (distance, tid).  Host-side test helper,
-    never on the product path."""
+    """part_merge_kernel restated for tests: greedy head merge of lists [(tids, dist), ...], each sorted by
+    (distance, tid) and -1 padded, ordered by (distance, tid).  For such lists the result is the k smallest pairs of
+    their union, whatever the grouping; lists in another order (a scan's gettuple order) are merged as they come.
+    Host-side test helper, never on the product path."""
     heads = [0] * len(lists)
     out_t, out_d = [], []
     for _ in range(k):
